@@ -273,6 +273,7 @@ def run_ours(args):
     torch.cuda.synchronize()
     D.barrier()
     ms_local = e0.elapsed_time(e1)
+    outputs = last_step_outputs(torch, p, local_rank, dst, stream) if args.dump_outputs and rank == 0 else None
     # sustained window next to the K-step figure (outside the timed region): back-to-back launches for >= 1 s, in batches of
     # 256 launches between two events; the clock sampler keeps running, so its summary covers a second of load
     sus_ms, sus_n = 0.0, 0
@@ -424,6 +425,12 @@ def run_ours(args):
                 "frac_of_measured_two_way_copy": (round(nvlink["gbs_per_gpu_per_direction"] / ce["gbs_per_gpu_per_direction"], 4) if ce.get("gbs_per_gpu_per_direction") else None),
                 "guide_one_way_peer_copy_gbs": NVLINK_GUIDE_ONE_WAY, "kernel": nvlink["kernel"],
                 "algorithmic_bytes_per_launch": nvlink["algorithmic_bytes_per_gpu_per_direction"], "traffic": None}
+    if outputs:
+        import numpy as np
+
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, arr in outputs.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), arr)
     if rank == 0:
         emit(line)
     # CPU-side wait: an NCCL barrier would park a spinning kernel on every waiting rank's GPU for as long as rank 0 works on its
@@ -436,6 +443,25 @@ def run_ours(args):
 
         td.destroy_process_group()
     return 0
+
+
+DUMP_WORDS = 1 << 22       # 4 Mi words of dst, 32 MiB as float64
+
+
+def last_step_outputs(torch, p, ordinal, dst, stream):
+    """What the timed copy handed its caller in the last step: dst (1 GiB), as the 32-bit words at a fixed seeded
+    sample of positions, and the sum64 / xor32 checksum of the whole buffer from the device, split into exact
+    32-bit halves.  float64 holds every uint32 exactly."""
+    import numpy as np
+
+    idx = np.sort(np.random.default_rng(0xB200).integers(0, dst.numel() // 4, DUMP_WORDS))
+    words = dst.view(torch.int32)[torch.from_numpy(idx).to(dst.device)].to(torch.int64) & 0xFFFFFFFF
+    part = torch.zeros(4, dtype=torch.int64, device=dst.device)
+    p.hbm_read(ordinal, dst.data_ptr(), dst.numel(), part.data_ptr(), stream)
+    torch.cuda.synchronize()
+    s, x = part[0].item() & 0xFFFFFFFFFFFFFFFF, part[1].item() & 0xFFFFFFFF
+    return {"dst_words_sample": words.cpu().numpy().astype(np.float64),
+            "dst_checksum": np.array([s & 0xFFFFFFFF, s >> 32, x], dtype=np.float64)}
 
 
 def nvlink_exchange(torch, D, p, local_rank, rank, world, stream, args):
@@ -676,7 +702,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-gemm", action="store_true", help="skip the GEMM roofline leg (about 20 s)")
     ap.add_argument("--no-probe-round", action="store_true", help="skip timing one full active-probe round")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the GPU arm")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

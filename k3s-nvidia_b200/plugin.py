@@ -268,7 +268,9 @@ class DevicePlugin:
                 log.info("inotify: %s created, restarting.", self.kubelet_socket)
                 try:
                     if self._server:
-                        self._server.stop(0)
+                        # gRPC unlinks the socket path when the old server's teardown completes, which can be after
+                        # serve() has bound the new one: wait for it, or the re-registered endpoint may vanish
+                        self._server.stop(0).wait()
                     self.serve()
                     self.register()
                 except Exception as e:  # noqa: BLE001

@@ -1,5 +1,8 @@
 import os
+import pathlib
+import shutil
 import sys
+import tempfile
 
 import pytest
 
@@ -15,7 +18,7 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session", autouse=True)
 def _built():
-    """Make sure the in-tree artefacts exist (the driver runs build() before the tests; this
+    """Make sure the in-tree artefacts exist (build() normally runs before the tests; this
     covers a bare `pytest`).  Never rebuilds what is already there."""
     need = [
         os.path.join(ROOT, "k3s-nvidia_b200", "libb200probe.so"),
@@ -29,3 +32,21 @@ def _built():
 
         g.build()
     yield
+
+
+# A unix socket path holds at most 107 bytes.  The deepest one the tests bind is <dir>/py/nvidia-gpu-shared.sock.
+_SOCK_DIR_MAX = 107 - len("/py/nvidia-gpu-shared.sock")
+
+
+@pytest.fixture
+def sock_dir(tmp_path):
+    """Directory for the kubelet and plugin sockets: tmp_path, unless a long TMPDIR makes it too deep for a
+    unix socket path, then a fresh short directory under /tmp that is removed afterwards."""
+    if len(str(tmp_path)) <= _SOCK_DIR_MAX:
+        yield tmp_path
+        return
+    d = tempfile.mkdtemp(prefix="b200probe-", dir="/tmp")
+    try:
+        yield pathlib.Path(d)
+    finally:
+        shutil.rmtree(d, ignore_errors=True)

@@ -9,13 +9,19 @@ from k3s_nvidia_b200 import config as cfgmod
 
 G = json.load(open(os.path.join(os.path.dirname(__file__), "golden", "golden.json")))
 VALUES = G["reference_inputs"]["values.yaml"]["text"]
+# sha256 of the files as UntouchedWagons/K3S-NVidia ships them, read from the original when the golden copies were made
+REFERENCE_SHA256 = {
+    "values.yaml": "91df8e3127981db3178d7fef23b7c91d2ddab62051d8264c44742852a8ee0d3b",
+    "nvidia-smi.yaml": "7f10e7f0ec783ef7ac1622abee2621d46d48adb937f002b5c2d29fda851853bc",
+    "jellyfin.yaml": "558fde9ce57e282d4cf5a1c23f1497c0fa0cc0cc1b4b5a82b61efa2bf61d0e8f",
+}
 
 
 def test_fixture_is_byte_identical_to_the_reference_when_present():
-    ref = "/root/reference/values.yaml"
-    assert hashlib.sha256(VALUES.encode()).hexdigest() == G["reference_inputs"]["values.yaml"]["sha256"]
-    if os.path.exists(ref):
-        assert open(ref, "rb").read() == VALUES.encode()
+    assert sorted(G["reference_inputs"]) == sorted(REFERENCE_SHA256)
+    for name, want in REFERENCE_SHA256.items():
+        doc = G["reference_inputs"][name]
+        assert hashlib.sha256(doc["text"].encode()).hexdigest() == doc["sha256"] == want, name
 
 
 def test_reference_values_parse_exactly():

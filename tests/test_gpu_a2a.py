@@ -23,6 +23,7 @@ def env():
     p = Probe()
     yield torch, p, _oracle.load()
     p.a2a_release()                  # the exchange context is resident between calls: hand the windows back
+    p.close()                        # b200probe_init is a no-op while a handle is open: later tests load their own NVML
 
 
 VARIANTS = {0: "auto", 1: "pull-tma", 2: "push-tma", 3: "push-direct", 4: "push-buf", 5: "mix-tma", 6: "push-stagger", 7: "push-sync"}

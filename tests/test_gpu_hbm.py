@@ -25,7 +25,9 @@ def env():
     from k3s_nvidia_b200.probe import Probe
 
     assert torch.cuda.is_available()
-    return torch, Probe(), _oracle.load()
+    p = Probe()
+    yield torch, p, _oracle.load()
+    p.close()                        # b200probe_init is a no-op while a handle is open: later tests load their own NVML
 
 
 def _dev_checksum(torch, p, t, nbytes, **tuning):

@@ -12,13 +12,13 @@ from test_native_plugin import BIN, Daemon, FakeKubelet
 pytestmark = pytest.mark.gpu
 
 
-def test_native_list_and_watch_matches_nvml_enumeration(tmp_path):
+def test_native_list_and_watch_matches_nvml_enumeration(sock_dir):
     from k3s_nvidia_b200.probe import Probe
 
     p = Probe()
     uuids = [p.device_info(i).uuid for i in range(p.device_count())]
     p.close()
-    d = str(tmp_path)
+    d = str(sock_dir)
     kubelet = FakeKubelet(d)
     kubelet.start()
     env = {k: v for k, v in os.environ.items() if not k.startswith("MOCK_NVML")}

@@ -98,7 +98,7 @@ def test_cuda_ordinals_resolve_by_uuid():
         p.close()
 
 
-def test_plugin_on_real_nvml(tmp_path):
+def test_plugin_on_real_nvml(sock_dir):
     """BASELINE config 5 plumbing: Register -> ListAndWatch (replicas x4 of the real UUIDs) ->
     Allocate one replica -> NVIDIA_VISIBLE_DEVICES is the real GPU's UUID."""
     import json
@@ -119,7 +119,7 @@ def test_plugin_on_real_nvml(tmp_path):
             got.set()
             return api.Empty()
 
-    d = str(tmp_path)
+    d = str(sock_dir)
     srv = grpc.server(futures.ThreadPoolExecutor(max_workers=2))
     api.add_servicer(srv, "Registration", Kubelet())
     srv.add_insecure_port("unix://" + os.path.join(d, "kubelet.sock"))

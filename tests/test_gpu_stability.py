@@ -20,7 +20,9 @@ def env():
     from k3s_nvidia_b200.probe import Probe
 
     assert torch.cuda.is_available()
-    return torch, Probe()
+    p = Probe()
+    yield torch, p
+    p.close()                        # b200probe_init is a no-op while a handle is open: later tests load their own NVML
 
 
 def spread(vals):

@@ -83,10 +83,10 @@ class PyDaemon(Daemon):
 
 
 @pytest.fixture(params=["native", "python"])
-def both_hosts(request, tmp_path, monkeypatch):
+def both_hosts(request, sock_dir, monkeypatch):
     """The same CLI contract for both hosts: flags, log lines the tests key on, signals."""
     monkeypatch.setenv("PYTHONPATH", ROOT + os.pathsep + os.environ.get("PYTHONPATH", ""))
-    d = str(tmp_path)
+    d = str(sock_dir)
     kubelet = FakeKubelet(d)
     kubelet.start()
     daemon = (Daemon if request.param == "native" else PyDaemon)(d, VALUES.raw_configs["default"])
@@ -99,8 +99,8 @@ def both_hosts(request, tmp_path, monkeypatch):
 
 
 @pytest.fixture
-def stack(tmp_path):
-    d = str(tmp_path)
+def stack(sock_dir):
+    d = str(sock_dir)
     kubelet = FakeKubelet(d)
     kubelet.start()
     daemon = Daemon(d, VALUES.raw_configs["default"])          # the config document exactly as the chart mounts it
@@ -193,8 +193,8 @@ def test_allocate_strips_replicas_and_dedupes(stack):
         assert e.value.code() == grpc.StatusCode.UNIMPLEMENTED
 
 
-def test_fail_requests_greater_than_one(tmp_path):
-    d = str(tmp_path)
+def test_fail_requests_greater_than_one(sock_dir):
+    d = str(sock_dir)
     kubelet = FakeKubelet(d)
     kubelet.start()
     daemon = Daemon(d, "version: v1\nsharing:\n  timeSlicing:\n    failRequestsGreaterThanOne: true\n    resources:\n    - name: nvidia.com/gpu\n      replicas: 4\n")
@@ -398,11 +398,11 @@ def test_hpack_decoder_against_libnghttp2_deflater():
     assert [json.loads(line) for line in out.splitlines()] == [{"error": "decode failed"}] * len(bad)
 
 
-def test_flow_control_large_device_list_and_large_unary_response(tmp_path):
+def test_flow_control_large_device_list_and_large_unary_response(sock_dir):
     """16 GPUs x 128 replicas = 2048 advertised devices: the ListAndWatch message (~110 KB) and a preferred
     allocation of 1500 IDs both exceed the 65,535-byte initial HTTP/2 windows, so DATA has to be cut into
     frames and wait for the peer's WINDOW_UPDATEs."""
-    d = str(tmp_path)
+    d = str(sock_dir)
     kubelet = FakeKubelet(d)
     kubelet.start()
     daemon = Daemon(d, "version: v1\nsharing:\n  timeSlicing:\n    resources:\n    - name: nvidia.com/gpu\n      replicas: 128\n",
@@ -809,7 +809,7 @@ def test_link_localisation_is_the_same_function_in_both_hosts():
 
 
 @pytest.mark.parametrize("host", ["native", "python"])
-def test_daemon_publishes_an_expiring_file_and_withdraws_it_on_sigterm(host, tmp_path, monkeypatch):
+def test_daemon_publishes_an_expiring_file_and_withdraws_it_on_sigterm(host, sock_dir, monkeypatch):
     """The active-probe runner inside the daemon (both hosts): first round at start-up writes features.d/b200probe with the
     expiry directive; SIGTERM wakes the runner out of its 600 s sleep at once (ADVICE r1: the native stop() could lose the
     wake-up and block for the whole interval), the verdicts are withdrawn and the process exits."""
@@ -818,7 +818,7 @@ def test_daemon_publishes_an_expiring_file_and_withdraws_it_on_sigterm(host, tmp
     if torch.cuda.is_available():
         pytest.skip("GPU present: the round would run the real probes")
     monkeypatch.setenv("PYTHONPATH", ROOT + os.pathsep + os.environ.get("PYTHONPATH", ""))
-    d = str(tmp_path)
+    d = str(sock_dir)
     kubelet = FakeKubelet(d)
     kubelet.start()
     cfg = os.path.join(d, "config.yaml")
@@ -1087,10 +1087,10 @@ def test_committed_huffman_table_is_what_libnghttp2_implements(tmp_path):
     assert out.read_text() == open(os.path.join(ROOT, "host", "cpp", "hpack_huffman.inc")).read()
 
 
-def test_unshared_config_and_index_strategy(tmp_path):
+def test_unshared_config_and_index_strategy(sock_dir):
     """No time-slicing: bare UUIDs are advertised and preferred allocation is required-first; deviceIDStrategy
     index makes Allocate answer with NVML indices (both as plugin.py does)."""
-    d = str(tmp_path)
+    d = str(sock_dir)
     kubelet = FakeKubelet(d)
     kubelet.start()
     daemon = Daemon(d, "version: v1\nflags:\n  migStrategy: none\n  plugin:\n    deviceIDStrategy: index\n", extra_env={"MOCK_NVML_DEVICES": "4"})

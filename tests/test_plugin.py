@@ -43,7 +43,7 @@ class FakeKubelet:
 
     def stop(self):
         if self.server:
-            self.server.stop(0)
+            self.server.stop(0).wait()         # teardown unlinks the socket path: finish it before a restart binds it again
 
     def plugin_channel(self):
         req = self.requests[-1]
@@ -51,11 +51,11 @@ class FakeKubelet:
 
 
 @pytest.fixture
-def stack(tmp_path, monkeypatch):
+def stack(sock_dir, monkeypatch):
     from k3s_nvidia_b200.probe import Probe
 
     monkeypatch.setenv("MOCK_NVML_DEVICES", "2")
-    d = str(tmp_path)
+    d = str(sock_dir)
     kubelet = FakeKubelet(d)
     kubelet.start()
     probe = Probe(_oracle.MOCK_NVML)
