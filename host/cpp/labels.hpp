@@ -172,10 +172,30 @@ inline Labels gemm_labels(const std::map<int, b200probe_gemm_result_t>& per_gpu,
     return out;
 }
 
+// Twin of labels.py memtest_labels: a mismatching word, uncorrected ECC errors during the run or a failed row remap fail
+// the verdict; corrected errors and a pending remap are published only (a pending remap does not affect further work).
+inline Labels memtest_labels(int idx, const b200probe_memtest_result_t& r) {
+    Labels out;
+    out[key(idx, "hbm-memtest-gib")] = rint_str((double)r.bytes_tested / (double)(1ull << 30));
+    out[key(idx, "hbm-memtest-bad-words")] = std::to_string((unsigned long long)r.bad_words);
+    if (r.ecc_corrected_delta >= 0) out[key(idx, "hbm-ecc-corrected-delta")] = std::to_string((long long)r.ecc_corrected_delta);
+    if (r.ecc_uncorrected_delta >= 0) out[key(idx, "hbm-ecc-uncorrected-delta")] = std::to_string((long long)r.ecc_uncorrected_delta);
+    if (r.ecc_after.remap_pending >= 0) out[key(idx, "hbm-row-remap-pending")] = b(r.ecc_after.remap_pending == 1);
+    if (r.ecc_after.remap_failure >= 0) out[key(idx, "hbm-row-remap-failed")] = b(r.ecc_after.remap_failure == 1);
+    out[key(idx, "hbm-memtest-healthy")] = b(r.bad_words == 0 && r.ecc_uncorrected_delta <= 0 && r.ecc_after.remap_failure != 1);
+    return out;
+}
+
+// B200PROBE_MEMTEST_FRACTION: share of each idle GPU's free memory the march test covers; unset or 0 = off
+inline double memtest_fraction() {
+    const double f = env_double("B200PROBE_MEMTEST_FRACTION", 0.0);
+    return f > 0.0 && f <= 1.0 ? f : 0.0;
+}
+
 // The one label manifests select on: every probe that has a verdict is healthy.  No verdict at all -> no gate label.
 inline void gate_label(Labels* l) {
     bool any = false, all = true;
-    for (const char* leaf : {"hbm-healthy", "nvlink-healthy", "gemm-healthy"}) {
+    for (const char* leaf : {"hbm-healthy", "nvlink-healthy", "gemm-healthy", "hbm-memtest-healthy"}) {
         auto it = l->find(key(leaf));
         if (it != l->end()) { any = true; all = all && it->second == "true"; }
     }
@@ -384,12 +404,32 @@ public:
                 }
             }
         }
+        if (const double fraction = memtest_fraction(); fraction > 0) {
+            for (const auto& d : infos) {
+                if (state[d.index] != "probed") continue;
+                b200probe_memtest_cfg_t cfg;
+                memset(&cfg, 0, sizeof(cfg));
+                cfg.fraction = fraction;
+                b200probe_memtest_result_t r;
+                const int rc = b200probe_hbm_memtest(d.index, &cfg, &r);
+                if (rc == B200PROBE_ENOMEM) {
+                    state[d.index] = "no-memory";
+                    plugin::logf("GPU %d: no device memory for the HBM memtest (tenants hold it): inconclusive", d.index);
+                } else if (rc) {
+                    plugin::logf("HBM memtest failed on GPU %d: %s", d.index, b200probe_strerror(rc));
+                    l[key(d.index, "hbm-memtest-healthy")] = "false";
+                } else {
+                    for (const auto& kv : memtest_labels(d.index, r)) l[kv.first] = kv.second;
+                }
+            }
+        }
         // GPUs that were skipped keep what their last measured round said
         for (const auto& d : infos) {
             l[key(d.index, "probe-state")] = state[d.index];
             if (state[d.index] != "probed") { carry(&l, d.index, "hbm-"); carry(&l, d.index, "gemm-"); }
         }
         aggregate(&l, "hbm-healthy");
+        aggregate(&l, "hbm-memtest-healthy");
         if (run_gemm_) aggregate(&l, "gemm-healthy");
         {
             bool have = false;

@@ -55,10 +55,12 @@ static int hpack_decode_stdin() {
 //   passive <gpu> <links_total> <links_active> <fabric_state> <fabric_status> <fabric_health_mask> [<active_mask>]
 //   a2a <G> <verified> <min_pair_gbs> <G egress> <G ingress> <G*G pair, row-major>
 //   a2ax <pair_source> <G ids>        (optional, after a2a: what the matrix holds and the NVML index of every position -> nvlink_localise)
+//   memtest <gpu> <bytes_tested> <bad_words> <ecc_corrected_delta> <ecc_uncorrected_delta> <remap_pending> <remap_failure>
 static int labels_from_stdin() {
     std::map<int, std::vector<b200probe_hbm_result_t>> hbm;
     std::map<int, b200probe_gemm_result_t> gemm;
     std::map<int, b200probe_nvlink_status_t> passive;
+    std::map<int, b200probe_memtest_result_t> memtest;
     bool have_a2a = false;
     b200probe_a2a_result_t rep;
     std::vector<double> pair;
@@ -95,6 +97,14 @@ static int labels_from_stdin() {
             pair.assign((size_t)(rep.g * rep.g), 0.0);
             for (auto& v : pair) in >> v;
             have_a2a = true;
+        } else if (kind == "memtest") {
+            int gpu; b200probe_memtest_result_t r;
+            memset(&r, 0, sizeof(r));
+            unsigned long long bytes, bad;
+            long long corr, unc;
+            in >> gpu >> bytes >> bad >> corr >> unc >> r.ecc_after.remap_pending >> r.ecc_after.remap_failure;
+            r.bytes_tested = bytes; r.bad_words = bad; r.ecc_corrected_delta = corr; r.ecc_uncorrected_delta = unc;
+            memtest[gpu] = r;
         } else if (kind == "a2ax") {
             in >> rep.pair_source;
             ids.assign((size_t)rep.g, 0);
@@ -107,6 +117,12 @@ static int labels_from_stdin() {
     if (!hbm.empty()) merge(labels::hbm_labels(hbm, th));
     if (!gemm.empty()) merge(labels::gemm_labels(gemm, th));
     merge(labels::nvlink_passive_labels(passive));
+    for (const auto& kv : memtest) merge(labels::memtest_labels(kv.first, kv.second));
+    if (!memtest.empty()) {
+        bool all = true;
+        for (const auto& kv : l) if (kv.first.size() > 20 && kv.first.compare(kv.first.size() - 20, 20, ".hbm-memtest-healthy") == 0) all = all && kv.second == "true";
+        l[labels::key("hbm-memtest-healthy")] = labels::b(all);
+    }
     if (have_a2a) {
         merge(labels::nvlink_labels(rep, pair, th, ids));
         if (!ids.empty()) merge(labels::nvlink_localise(rep, pair, ids, passive));

@@ -236,6 +236,65 @@ func HBMVerify(ordinal int, devPtr unsafe.Pointer, bytes uint64, seed uint32) (s
 	return uint64(s), uint32(x), uint64(b), uint64(f), err
 }
 
+// ECCStatus mirrors b200probe_ecc_status_t; every field is -1 when NVML cannot report it.
+type ECCStatus struct {
+	ECCMode                               int
+	CorrectedVolatile, UncorrectedVolatile int64
+	RemapCorrectedRows, RemapUncorrectedRows int
+	RemapPending, RemapFailure            int
+}
+
+func eccOf(e *C.b200probe_ecc_status_t) ECCStatus {
+	return ECCStatus{int(e.ecc_mode), int64(e.corrected_volatile), int64(e.uncorrected_volatile), int(e.remap_corrected_rows),
+		int(e.remap_uncorrected_rows), int(e.remap_pending), int(e.remap_failure)}
+}
+
+// HBMECC reads the ECC mode, the volatile corrected / uncorrected totals and the row remapper's state of NVML device idx.
+func HBMECC(idx int) (ECCStatus, error) {
+	var e C.b200probe_ecc_status_t
+	err := check(C.b200probe_hbm_ecc(C.int(idx), &e))
+	return eccOf(&e), err
+}
+
+// MemtestElement runs one march element on a device buffer of CUDA device `ordinal` (flags: 1 verify, 2 write) and
+// returns the mismatching words, the lowest mismatching word index (^0 when none) and the OR of got ^ want.
+func MemtestElement(ordinal int, devPtr unsafe.Pointer, bytes, baseWord uint64, flags int, expectSeed, writeSeed uint32) (bad, first uint64, bits uint32, err error) {
+	runtime.LockOSThread()
+	defer runtime.UnlockOSThread()
+	var b, f C.uint64_t
+	var x C.uint32_t
+	err = check(C.b200probe_memtest_element(C.int(ordinal), devPtr, C.uint64_t(bytes), C.uint64_t(baseWord), C.int(flags), C.uint32_t(expectSeed),
+		C.uint32_t(writeSeed), &b, &f, &x))
+	return uint64(b), uint64(f), uint32(x), err
+}
+
+// MemtestResult mirrors b200probe_memtest_result_t.
+type MemtestResult struct {
+	BytesTested, FreeBefore, Total             uint64
+	Chunks, Passes                             int
+	AllocMs, TestMs, GBs                       float64
+	BadWords, FirstBadWord                     uint64
+	BadBits                                    uint32
+	FirstBadElement                            int
+	ECCCorrectedDelta, ECCUncorrectedDelta     int64
+	ECCAfter                                   ECCStatus
+}
+
+// HBMMemtest runs the march test over fraction x the free memory of NVML device idx (0 = 0.9) and frees everything
+// before it returns. rc -10 (ErrNoMem) = inconclusive: tenants hold the memory.
+func HBMMemtest(idx int, fraction float64, passes int) (MemtestResult, error) {
+	runtime.LockOSThread()
+	defer runtime.UnlockOSThread()
+	var cfg C.b200probe_memtest_cfg_t
+	cfg.fraction = C.double(fraction)
+	cfg.passes = C.int(passes)
+	var r C.b200probe_memtest_result_t
+	err := check(C.b200probe_hbm_memtest(C.int(idx), &cfg, &r))
+	return MemtestResult{uint64(r.bytes_tested), uint64(r.free_before), uint64(r.total), int(r.chunks), int(r.passes), float64(r.alloc_ms),
+		float64(r.test_ms), float64(r.gbs), uint64(r.bad_words), uint64(r.first_bad_word), uint32(r.bad_bits), int(r.first_bad_element),
+		int64(r.ecc_corrected_delta), int64(r.ecc_uncorrected_delta), eccOf(&r.ecc_after)}, err
+}
+
 // HostAlloc returns page-locked host memory for HBMCopyHost (C-owned: release with HostFree, never the Go GC).
 func HostAlloc(bytes uint64) (unsafe.Pointer, error) {
 	var p unsafe.Pointer

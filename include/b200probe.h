@@ -18,6 +18,9 @@
  *   b200probe_hbm_*         -> NEW: no reference counterpart (SURVEY.md §8a row a11)
  *   b200probe_a2a_*         -> NEW: row a12
  *   b200probe_gemm*         -> NEW: row a13
+ *   b200probe_hbm_memtest,
+ *   b200probe_memtest_element,
+ *   b200probe_hbm_ecc       -> NEW: HBM integrity (DESIGN.md §4.4)
  *
  * Error convention: 0 = OK; negative = library error (B200PROBE_E*); positive = a foreign status
  * tagged by range: 1000+cudaError_t, 2000+nvmlReturn_t, 3000+ncclResult_t.
@@ -211,6 +214,65 @@ int b200probe_hbm_copy_host(int cuda_ordinal, const void* src_host, void* dst_ho
 /* Page-locked host memory for the entry above (cudaHostAlloc, portable across devices). */
 int b200probe_host_alloc(uint64_t bytes, void** ptr);
 int b200probe_host_free(void* ptr);
+
+/* ---- HBM integrity: march test over the free memory, joined with NVML ECC / row-remap state ------- */
+/* Passive side.  Every field is -1 when NVML does not support or does not export the query. */
+typedef struct b200probe_ecc_status {
+    int      ecc_mode;              /* nvmlDeviceGetEccMode, current: 1 enabled, 0 disabled          */
+    int64_t  corrected_volatile;    /* nvmlDeviceGetTotalEccErrors(CORRECTED, VOLATILE): since driver load */
+    int64_t  uncorrected_volatile;  /* nvmlDeviceGetTotalEccErrors(UNCORRECTED, VOLATILE)           */
+    int      remap_corrected_rows;  /* nvmlDeviceGetRemappedRows: rows remapped for corrected errors */
+    int      remap_uncorrected_rows;/* … for uncorrected errors                                     */
+    int      remap_pending;         /* 1 = a remap waits for the next GPU reset                      */
+    int      remap_failure;         /* 1 = a remap failed (no spare row left)                        */
+} b200probe_ecc_status_t;
+int b200probe_hbm_ecc(int idx, b200probe_ecc_status_t* out);
+
+/* One march element over a device buffer of device cuda_ordinal, for every u32 word i:
+ *   VERIFY: compare buf[i] with pattern(base_word + i, expect_seed);
+ *   WRITE : then store pattern(base_word + i, write_seed) in place.
+ * base_word places the buffer in a larger tested space (address-in-address across chunks); the
+ * complement of a pattern is the pattern under seed ^ 0xFFFFFFFF.  bytes a multiple of 4, buf
+ * 16-byte aligned.  Mismatches: count, lowest global word index (~0 when none) and the OR of
+ * got ^ want over all of them.  Synchronous; holds no device memory after it returns. */
+#define B200PROBE_MEMTEST_VERIFY 1
+#define B200PROBE_MEMTEST_WRITE  2
+int b200probe_memtest_element(int cuda_ordinal, void* buf, uint64_t bytes, uint64_t base_word, int flags,
+                              uint32_t expect_seed, uint32_t write_seed,
+                              uint64_t* bad_words, uint64_t* first_bad_word, uint32_t* bad_bits);
+
+typedef struct b200probe_memtest_cfg {
+    double   fraction;              /* of cudaMemGetInfo's free bytes, in (0, 1]; 0 = 0.9          */
+    uint64_t max_bytes;             /* cap on the bytes tested; 0 = none                           */
+    uint64_t min_bytes;             /* fewer bytes allocated -> B200PROBE_ENOMEM; 0 = one byte      */
+    uint64_t chunk_bytes;           /* allocation unit, multiple of 4096; 0 = 1 GiB                 */
+    int      passes;                /* 0 = 1                                                       */
+    uint32_t seed;                  /* s0; 0 = 0xB200.  s1 = s0 ^ 0x5A5A5A5A                       */
+} b200probe_memtest_cfg_t;
+
+typedef struct b200probe_memtest_result {
+    uint64_t bytes_tested;
+    int      chunks, passes;
+    uint64_t free_before, total;    /* cudaMemGetInfo before the allocation                         */
+    double   alloc_ms, test_ms;     /* allocation (host clock); all elements of all passes (events) */
+    double   gbs;                   /* algorithmic bytes (6 x bytes_tested per pass) / test_ms      */
+    uint64_t bad_words;             /* mismatching words, summed over the verifying elements        */
+    uint64_t first_bad_word;        /* lowest mismatching word index (in the tested space) of the
+                                       first element that saw one; ~0 when none                    */
+    uint32_t bad_bits;              /* OR of got ^ want over every mismatch                          */
+    int      first_bad_element;     /* 1, 2 or 3 (E1..E3) of that element; -1 when none            */
+    int64_t  ecc_corrected_delta;   /* volatile ECC totals after - before; -1 when unreadable       */
+    int64_t  ecc_uncorrected_delta;
+    b200probe_ecc_status_t ecc_after;
+} b200probe_memtest_result_t;
+
+/* The HBM integrity probe on NVML device idx: ECC snapshot; allocate fraction x free (capped by
+ * max_bytes) in chunk_bytes pieces, stopping at the first failed allocation; march
+ *   E0 write P(s0); E1 verify P(s0), write ~P(s0); E2 verify ~P(s0), write P(s1); E3 verify P(s1)
+ * with every element over all chunks before the next one, `passes` times; ECC snapshot; free.
+ * Nothing stays allocated after the call, on any path.  Less than min_bytes allocated returns
+ * B200PROBE_ENOMEM (a resource verdict, not a fault); mismatches are results, not errors. */
+int b200probe_hbm_memtest(int idx, const b200probe_memtest_cfg_t* cfg, b200probe_memtest_result_t* out);
 
 /* ---- NVLink all-to-all (row a12) --------------------------------------------------------------- */
 #define B200PROBE_A2A_PEER_ALL    0   /* our peer-memory kernel, all pairs concurrently            */

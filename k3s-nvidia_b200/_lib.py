@@ -20,6 +20,7 @@ VARIANT_TMA, VARIANT_DIRECT = 0, 1
 A2A_PEER_ALL, A2A_PEER_PAIR, A2A_NCCL, A2A_CE = 0, 1, 2, 3
 PAIR_SHARE, PAIR_ISOLATED, PAIR_STEPPED = 0, 1, 2
 GEMM_EXACT, GEMM_UNIFORM = 0, 1
+MEMTEST_VERIFY, MEMTEST_WRITE = 1, 2
 A2A_AUTO, A2A_PULL_TMA, A2A_PUSH_TMA, A2A_PUSH_DIRECT, A2A_PUSH_BUF, A2A_MIX_TMA, A2A_PUSH_STAGGER, A2A_PUSH_SYNC = 0, 1, 2, 3, 4, 5, 6, 7
 A2A_SYNC_BYTES = 4096
 NVML_ERROR_TIMEOUT = 10
@@ -181,6 +182,49 @@ class GemmResult(C.Structure):
     ]
 
 
+class EccStatus(C.Structure):
+    _fields_ = [
+        ("ecc_mode", C.c_int),
+        ("corrected_volatile", C.c_int64),
+        ("uncorrected_volatile", C.c_int64),
+        ("remap_corrected_rows", C.c_int),
+        ("remap_uncorrected_rows", C.c_int),
+        ("remap_pending", C.c_int),
+        ("remap_failure", C.c_int),
+    ]
+
+
+class MemtestCfg(C.Structure):
+    _fields_ = [
+        ("fraction", C.c_double),
+        ("max_bytes", C.c_uint64),
+        ("min_bytes", C.c_uint64),
+        ("chunk_bytes", C.c_uint64),
+        ("passes", C.c_int),
+        ("seed", C.c_uint32),
+    ]
+
+
+class MemtestResult(C.Structure):
+    _fields_ = [
+        ("bytes_tested", C.c_uint64),
+        ("chunks", C.c_int),
+        ("passes", C.c_int),
+        ("free_before", C.c_uint64),
+        ("total", C.c_uint64),
+        ("alloc_ms", C.c_double),
+        ("test_ms", C.c_double),
+        ("gbs", C.c_double),
+        ("bad_words", C.c_uint64),
+        ("first_bad_word", C.c_uint64),
+        ("bad_bits", C.c_uint32),
+        ("first_bad_element", C.c_int),
+        ("ecc_corrected_delta", C.c_int64),
+        ("ecc_uncorrected_delta", C.c_int64),
+        ("ecc_after", EccStatus),
+    ]
+
+
 _P = C.POINTER
 _vp = C.c_void_p
 
@@ -208,6 +252,10 @@ SIGNATURES = {
     "b200probe_hbm_read": (C.c_int, [C.c_int, _vp, C.c_uint64, _vp, _P(HbmCfg), _vp]),
     "b200probe_hbm_copy_host": (C.c_int, [C.c_int, _vp, _vp, C.c_uint64, _P(C.c_uint64), _P(C.c_uint32)]),
     "b200probe_hbm_verify": (C.c_int, [C.c_int, _vp, C.c_uint64, C.c_uint32, _P(C.c_uint64), _P(C.c_uint32), _P(C.c_uint64), _P(C.c_uint64)]),
+    "b200probe_hbm_ecc": (C.c_int, [C.c_int, _P(EccStatus)]),
+    "b200probe_memtest_element": (C.c_int, [C.c_int, _vp, C.c_uint64, C.c_uint64, C.c_int, C.c_uint32, C.c_uint32, _P(C.c_uint64), _P(C.c_uint64),
+                                            _P(C.c_uint32)]),
+    "b200probe_hbm_memtest": (C.c_int, [C.c_int, _P(MemtestCfg), _P(MemtestResult)]),
     "b200probe_host_alloc": (C.c_int, [C.c_uint64, _P(_vp)]),
     "b200probe_host_free": (C.c_int, [_vp]),
     "b200probe_nvlink_a2a": (C.c_int, [_P(C.c_int), C.c_int, _P(A2aCfg), _P(C.c_double), _P(A2aResult)]),

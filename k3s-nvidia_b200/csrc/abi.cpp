@@ -46,6 +46,9 @@ struct Nvml {
     nvmlReturn_t (*DeviceGetGpuFabricInfoV)(nvmlDevice_t, nvmlGpuFabricInfoV_t*);            // optional
     nvmlReturn_t (*DeviceGetComputeRunningProcesses_v3)(nvmlDevice_t, unsigned int*, nvmlProcessInfo_t*);   // optional
     nvmlReturn_t (*DeviceGetUtilizationRates)(nvmlDevice_t, nvmlUtilization_t*);                          // optional
+    nvmlReturn_t (*DeviceGetEccMode)(nvmlDevice_t, nvmlEnableState_t*, nvmlEnableState_t*);                // optional
+    nvmlReturn_t (*DeviceGetTotalEccErrors)(nvmlDevice_t, nvmlMemoryErrorType_t, nvmlEccCounterType_t, unsigned long long*);   // optional
+    nvmlReturn_t (*DeviceGetRemappedRows)(nvmlDevice_t, unsigned int*, unsigned int*, unsigned int*, unsigned int*);         // optional
 };
 
 struct Device {
@@ -367,6 +370,9 @@ int b200probe_init(const char* path) {
     sym(lib, "nvmlDeviceGetGpuFabricInfoV", n.DeviceGetGpuFabricInfoV, false);
     sym(lib, "nvmlDeviceGetComputeRunningProcesses_v3", n.DeviceGetComputeRunningProcesses_v3, false);
     sym(lib, "nvmlDeviceGetUtilizationRates", n.DeviceGetUtilizationRates, false);
+    sym(lib, "nvmlDeviceGetEccMode", n.DeviceGetEccMode, false);
+    sym(lib, "nvmlDeviceGetTotalEccErrors", n.DeviceGetTotalEccErrors, false);
+    sym(lib, "nvmlDeviceGetRemappedRows", n.DeviceGetRemappedRows, false);
     if (!ok) { dlclose(lib); return B200PROBE_ENVML; }
     nvmlReturn_t r = n.Init_v2();
     if (r != NVML_SUCCESS) { b200::set_error("nvmlInit_v2: %s", n.ErrorString(r)); dlclose(lib); return nvml_rc(r); }
@@ -591,6 +597,33 @@ int b200probe_device_busy(int idx, b200probe_busy_t* out) {
     nvmlMemory_t mem;
     if (g.nvml.DeviceGetMemoryInfo(h, &mem) == NVML_SUCCESS) out->mem_used = mem.used;
     out->busy = (out->compute_procs > 0 || out->util_gpu_pct >= B200PROBE_BUSY_UTIL_PCT) ? 1 : 0;
+    return 0;
+}
+
+// Passive half of the HBM integrity probe: ECC mode (nvml.h:6249), the volatile corrected / uncorrected totals (:6349)
+// and the row remapper's state (:7730).  b200probe_hbm_memtest takes this snapshot before and after its march.
+int b200probe_hbm_ecc(int idx, b200probe_ecc_status_t* out) {
+    if (!out) return B200PROBE_EINVAL;
+    Lock l;
+    if (!g.inited) return B200PROBE_ENOTINIT;
+    if (idx < 0 || idx >= (int)g.devs.size()) return B200PROBE_ERANGE;
+    out->ecc_mode = out->remap_corrected_rows = out->remap_uncorrected_rows = out->remap_pending = out->remap_failure = -1;
+    out->corrected_volatile = out->uncorrected_volatile = -1;
+    nvmlDevice_t h = g.devs[idx].h;
+    nvmlEnableState_t cur, pend;
+    if (g.nvml.DeviceGetEccMode && g.nvml.DeviceGetEccMode(h, &cur, &pend) == NVML_SUCCESS) out->ecc_mode = cur == NVML_FEATURE_ENABLED ? 1 : 0;
+    unsigned long long v;
+    if (g.nvml.DeviceGetTotalEccErrors) {
+        if (g.nvml.DeviceGetTotalEccErrors(h, NVML_MEMORY_ERROR_TYPE_CORRECTED, NVML_VOLATILE_ECC, &v) == NVML_SUCCESS) out->corrected_volatile = (int64_t)v;
+        if (g.nvml.DeviceGetTotalEccErrors(h, NVML_MEMORY_ERROR_TYPE_UNCORRECTED, NVML_VOLATILE_ECC, &v) == NVML_SUCCESS) out->uncorrected_volatile = (int64_t)v;
+    }
+    unsigned corr, unc, pending, failure;
+    if (g.nvml.DeviceGetRemappedRows && g.nvml.DeviceGetRemappedRows(h, &corr, &unc, &pending, &failure) == NVML_SUCCESS) {
+        out->remap_corrected_rows = (int)corr;
+        out->remap_uncorrected_rows = (int)unc;
+        out->remap_pending = pending ? 1 : 0;
+        out->remap_failure = failure ? 1 : 0;
+    }
     return 0;
 }
 

@@ -195,10 +195,35 @@ def gemm_labels(per_gpu: Dict[int, object], th: Thresholds) -> Dict[str, str]:
     return out
 
 
+def memtest_labels(idx: int, r) -> Dict[str, str]:
+    """r: probe.MemtestReport of GPU idx.  The verdict fails on a mismatching word, on uncorrected ECC errors during the
+    run and on a failed row remap.  Corrected errors and a pending remap are published only: ECC fixed the data, and a
+    pending remap does not affect further work until the next GPU reset applies it (nvml.h:7730)."""
+    k = f"{PREFIX}gpu{idx}."
+    out = {k + "hbm-memtest-gib": str(int(round(r.bytes_tested / float(1 << 30)))), k + "hbm-memtest-bad-words": str(r.bad_words)}
+    if r.ecc_corrected_delta >= 0:
+        out[k + "hbm-ecc-corrected-delta"] = str(r.ecc_corrected_delta)
+    if r.ecc_uncorrected_delta >= 0:
+        out[k + "hbm-ecc-uncorrected-delta"] = str(r.ecc_uncorrected_delta)
+    if r.remap_pending >= 0:
+        out[k + "hbm-row-remap-pending"] = _b(r.remap_pending == 1)
+    if r.remap_failure >= 0:
+        out[k + "hbm-row-remap-failed"] = _b(r.remap_failure == 1)
+    out[k + "hbm-memtest-healthy"] = _b(r.bad_words == 0 and r.ecc_uncorrected_delta <= 0 and r.remap_failure != 1)
+    return out
+
+
+def memtest_fraction() -> float:
+    """B200PROBE_MEMTEST_FRACTION: share of each idle GPU's free memory the march test covers; unset or 0 = off."""
+    f = _env_float("B200PROBE_MEMTEST_FRACTION", 0.0)
+    return f if 0.0 < f <= 1.0 else 0.0
+
+
 def gate_label(labels: Dict[str, str]) -> Dict[str, str]:
     """The one label manifests select on: every probe that has a verdict is healthy.  No verdict at all (every GPU
     busy since the daemon started) -> no gate label: unknown is not healthy."""
-    parts = [v for k, v in labels.items() if k in (f"{PREFIX}hbm-healthy", f"{PREFIX}nvlink-healthy", f"{PREFIX}gemm-healthy")]
+    parts = [v for k, v in labels.items()
+             if k in (f"{PREFIX}hbm-healthy", f"{PREFIX}nvlink-healthy", f"{PREFIX}gemm-healthy", f"{PREFIX}hbm-memtest-healthy")]
     return {f"{PREFIX}healthy": _b(all(v == "true" for v in parts))} if parts else {}
 
 
@@ -439,6 +464,23 @@ class ActiveProbeRunner:
                 labels.update({k: v for k, v in got.items() if _GPU_KEY.match(k)})
                 if got.get(f"{PREFIX}gpu{idx}.gemm-healthy") == "true":
                     self.cal.offer(f"gemm-tflops.{uuid}", r.tflops_median, GEMM_MEASURED_TFLOPS)
+        fraction = memtest_fraction()
+        if fraction > 0:
+            for d in infos:
+                if state[d.index] != "probed":
+                    continue
+                try:
+                    labels.update(memtest_labels(d.index, self.probe.hbm_memtest(d.index, fraction=fraction)))
+                except ProbeError as e:
+                    if e.rc == ENOMEM:
+                        state[d.index] = "no-memory"
+                        log.warning("GPU %d: no device memory for the HBM memtest (tenants hold it): inconclusive", d.index)
+                        continue
+                    log.error("HBM memtest failed on GPU %d: %s", d.index, e)
+                    labels[f"{PREFIX}gpu{d.index}.hbm-memtest-healthy"] = "false"
+                except Exception as e:  # noqa: BLE001
+                    log.error("HBM memtest failed on GPU %d: %s", d.index, e)
+                    labels[f"{PREFIX}gpu{d.index}.hbm-memtest-healthy"] = "false"
         # GPUs that were skipped keep what their last measured round said
         for d in infos:
             labels[f"{PREFIX}gpu{d.index}.probe-state"] = state[d.index]
@@ -446,6 +488,7 @@ class ActiveProbeRunner:
                 self._carry(labels, d.index, "hbm-")
                 self._carry(labels, d.index, "gemm-")
         self._aggregate(labels, "hbm-healthy")
+        self._aggregate(labels, "hbm-memtest-healthy")
         if self.run_gemm:
             self._aggregate(labels, "gemm-healthy")
         copies = [float(v) for k, v in labels.items() if (m := _GPU_KEY.match(k)) and m.group(2) == "hbm-copy-gbs"]

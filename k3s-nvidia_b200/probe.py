@@ -86,6 +86,29 @@ class GemmReport:
 
 
 @dataclass
+class MemtestReport:
+    """b200probe_memtest_result_t; ECC and remap fields are -1 where NVML cannot report them."""
+    bytes_tested: int
+    chunks: int
+    passes: int
+    free_before: int
+    total: int
+    alloc_ms: float
+    test_ms: float
+    gbs: float
+    bad_words: int
+    first_bad_word: int
+    bad_bits: int
+    first_bad_element: int
+    ecc_corrected_delta: int
+    ecc_uncorrected_delta: int
+    remap_corrected_rows: int
+    remap_uncorrected_rows: int
+    remap_pending: int
+    remap_failure: int
+
+
+@dataclass
 class HealthEvent:
     rc_wait: int
     event_type: int
@@ -230,6 +253,28 @@ class Probe:
         self._check(self.lib.b200probe_hbm_verify(ordinal, ptr, nbytes, seed, C.byref(s64), C.byref(x32), C.byref(bad), C.byref(first)),
                     "hbm_verify")
         return s64.value, x32.value, bad.value, first.value
+
+    # -- HBM integrity ---------------------------------------------------------------------------
+    def memtest_element(self, ordinal: int, ptr: int, nbytes: int, base_word: int, flags: int, expect_seed: int, write_seed: int):
+        """One march element on a device buffer -> (bad_words, first_bad_word, bad_bits)."""
+        bad, first, bits = C.c_uint64(), C.c_uint64(), C.c_uint32()
+        self._check(self.lib.b200probe_memtest_element(ordinal, ptr, nbytes, base_word, flags, expect_seed & 0xFFFFFFFF, write_seed & 0xFFFFFFFF,
+                                                       C.byref(bad), C.byref(first), C.byref(bits)), "memtest_element")
+        return bad.value, first.value, bits.value
+
+    def hbm_ecc(self, idx: int) -> dict:
+        st = L.EccStatus()
+        self._check(self.lib.b200probe_hbm_ecc(idx, C.byref(st)), "hbm_ecc")
+        return {f: getattr(st, f) for f, _ in L.EccStatus._fields_}
+
+    def hbm_memtest(self, idx: int = 0, *, fraction=0.0, max_bytes=0, min_bytes=0, chunk_bytes=0, passes=0, seed=0) -> MemtestReport:
+        cfg = L.MemtestCfg(fraction, max_bytes, min_bytes, chunk_bytes, passes, seed)
+        r = L.MemtestResult()
+        self._check(self.lib.b200probe_hbm_memtest(idx, C.byref(cfg), C.byref(r)), "hbm_memtest")
+        e = r.ecc_after
+        return MemtestReport(r.bytes_tested, r.chunks, r.passes, r.free_before, r.total, r.alloc_ms, r.test_ms, r.gbs, r.bad_words,
+                             r.first_bad_word, r.bad_bits, r.first_bad_element, r.ecc_corrected_delta, r.ecc_uncorrected_delta,
+                             e.remap_corrected_rows, e.remap_uncorrected_rows, e.remap_pending, e.remap_failure)
 
     def host_alloc(self, nbytes: int):
         """Pinned host buffer as a numpy uint8 array (free with host_free(arr))."""
