@@ -39,6 +39,9 @@ static const double kHbmNominal = 8000.0, kHbmMeasured = 6565.8;            // n
 static const double kNvlinkNominal = 900.0;
 static const double kNvlinkHealthyPair = 692.0, kNvlinkHealthyBox = 700.0;  // profiles/a2a_tune_r01_2gpu.txt; profiles/a2a_sync_relaxed_r01_g8.txt
 static const double kGemmMeasured = 1670.2;
+// cuBLASLt FP8 (torch._scaled_mm, E4M3 x E4M3, scales 1.0, bf16 out) at 8192^3, burst median on a B200 at its 1000 W power
+// limit, EXACT operands (profiles/gemm_fp8_bench_r01.txt); twin of labels.py GEMM_FP8_MEASURED_TFLOPS
+static const double kGemmFp8Measured = 3268.0;
 
 using Labels = std::map<std::string, std::string>;
 
@@ -54,6 +57,7 @@ struct Thresholds {
     double hbm_min_gbs = env_double("B200PROBE_HBM_MIN_GBS", 0.90 * kHbmMeasured);
     double nvlink_min_gbs = env_double("B200PROBE_NVLINK_MIN_GBS", 0.0);     // 0 = 97 % of the healthy figure for the number of GPUs exchanged
     double gemm_min_tflops = env_double("B200PROBE_GEMM_MIN_TFLOPS", 0.70 * kGemmMeasured);
+    double gemm_fp8_min_tflops = env_double("B200PROBE_GEMM_FP8_MIN_TFLOPS", 0.70 * kGemmFp8Measured);
     uint64_t verdict_min_bytes = 256ull << 20;                                // sizes below L2 are cache-resident: never used for the verdict
 };
 
@@ -172,6 +176,28 @@ inline Labels gemm_labels(const std::map<int, b200probe_gemm_result_t>& per_gpu,
     return out;
 }
 
+// Twin of labels.py gemm_fp8_labels: the bf16 GEMM's rules on the FP8 probe's own keys and threshold
+inline Labels gemm_fp8_labels(const std::map<int, b200probe_gemm_result_t>& per_gpu, const Thresholds& th) {
+    Labels out;
+    bool all_ok = true;
+    for (const auto& kv : per_gpu) {
+        const auto& r = kv.second;
+        const bool ok = r.verified == 1 && r.tflops_median >= th.gemm_fp8_min_tflops;
+        out[key(kv.first, "gemm-fp8-tflops")] = rint_str(r.tflops_median);
+        out[key(kv.first, "gemm-fp8-data-ok")] = b(r.verified == 1);
+        out[key(kv.first, "gemm-fp8-healthy")] = b(ok);
+        all_ok = all_ok && ok;
+    }
+    out[key("gemm-fp8-healthy")] = b(all_ok && !per_gpu.empty());
+    return out;
+}
+
+// B200PROBE_GEMM_FP8=1: every idle GPU also runs the FP8 tensor-core probe; unset or 0 = off
+inline bool gemm_fp8_enabled() {
+    const char* e = getenv("B200PROBE_GEMM_FP8");
+    return e && *e && strcmp(e, "0") != 0;
+}
+
 // Twin of labels.py memtest_labels: a mismatching word, uncorrected ECC errors during the run or a failed row remap fail
 // the verdict; corrected errors and a pending remap are published only (a pending remap does not affect further work).
 inline Labels memtest_labels(int idx, const b200probe_memtest_result_t& r) {
@@ -195,7 +221,7 @@ inline double memtest_fraction() {
 // The one label manifests select on: every probe that has a verdict is healthy.  No verdict at all -> no gate label.
 inline void gate_label(Labels* l) {
     bool any = false, all = true;
-    for (const char* leaf : {"hbm-healthy", "nvlink-healthy", "gemm-healthy", "hbm-memtest-healthy"}) {
+    for (const char* leaf : {"hbm-healthy", "nvlink-healthy", "gemm-healthy", "hbm-memtest-healthy", "gemm-fp8-healthy"}) {
         auto it = l->find(key(leaf));
         if (it != l->end()) { any = true; all = all && it->second == "true"; }
     }
@@ -351,6 +377,7 @@ public:
             state[d.index] = (!ignore_tenants && b200probe_device_busy(d.index, &busy) == 0 && busy.busy) ? "busy" : "probed";
         }
         const bool explicit_hbm = getenv("B200PROBE_HBM_MIN_GBS") != nullptr, explicit_gemm = getenv("B200PROBE_GEMM_MIN_TFLOPS") != nullptr;
+        const bool explicit_gemm_fp8 = getenv("B200PROBE_GEMM_FP8_MIN_TFLOPS") != nullptr;
 
         for (const auto& d : infos) {
             if (state[d.index] != "probed") continue;
@@ -404,6 +431,33 @@ public:
                 }
             }
         }
+        if (gemm_fp8_enabled()) {
+            for (const auto& d : infos) {
+                if (state[d.index] != "probed") continue;
+                b200probe_gemm_cfg_t cfg;
+                memset(&cfg, 0, sizeof(cfg));
+                cfg.warmup = 2; cfg.reps = 5;
+                b200probe_gemm_result_t r;
+                const int rc = b200probe_gemm_fp8(d.index, &cfg, &r);
+                if (rc == B200PROBE_ENOMEM) {
+                    state[d.index] = "no-memory";
+                    plugin::logf("GPU %d: no device memory for the FP8 GEMM probe (tenants hold it): inconclusive", d.index);
+                } else if (rc) {
+                    plugin::logf("FP8 GEMM probe failed on GPU %d: %s", d.index, b200probe_strerror(rc));
+                    l[key(d.index, "gemm-fp8-healthy")] = "false";
+                } else {
+                    Thresholds th = th_;
+                    const std::string ck = std::string("gemm-fp8-tflops.") + d.uuid;
+                    if (!explicit_gemm_fp8) th.gemm_fp8_min_tflops = 0.70 * cal_.get(ck, kGemmFp8Measured);
+                    std::map<int, b200probe_gemm_result_t> one;
+                    one[d.index] = r;
+                    Labels gl = gemm_fp8_labels(one, th);
+                    for (const auto& kv : gl) if (is_gpu_key(kv.first)) l[kv.first] = kv.second;
+                    auto h = gl.find(key(d.index, "gemm-fp8-healthy"));
+                    if (h != gl.end() && h->second == "true") cal_.offer(ck, r.tflops_median, kGemmFp8Measured);
+                }
+            }
+        }
         if (const double fraction = memtest_fraction(); fraction > 0) {
             for (const auto& d : infos) {
                 if (state[d.index] != "probed") continue;
@@ -430,6 +484,7 @@ public:
         }
         aggregate(&l, "hbm-healthy");
         aggregate(&l, "hbm-memtest-healthy");
+        aggregate(&l, "gemm-fp8-healthy");
         if (run_gemm_) aggregate(&l, "gemm-healthy");
         {
             bool have = false;

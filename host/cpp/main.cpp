@@ -55,10 +55,11 @@ static int hpack_decode_stdin() {
 //   passive <gpu> <links_total> <links_active> <fabric_state> <fabric_status> <fabric_health_mask> [<active_mask>]
 //   a2a <G> <verified> <min_pair_gbs> <G egress> <G ingress> <G*G pair, row-major>
 //   a2ax <pair_source> <G ids>        (optional, after a2a: what the matrix holds and the NVML index of every position -> nvlink_localise)
+//   gemm_fp8 <gpu> <tflops_median> <verified>
 //   memtest <gpu> <bytes_tested> <bad_words> <ecc_corrected_delta> <ecc_uncorrected_delta> <remap_pending> <remap_failure>
 static int labels_from_stdin() {
     std::map<int, std::vector<b200probe_hbm_result_t>> hbm;
-    std::map<int, b200probe_gemm_result_t> gemm;
+    std::map<int, b200probe_gemm_result_t> gemm, gemm_fp8;
     std::map<int, b200probe_nvlink_status_t> passive;
     std::map<int, b200probe_memtest_result_t> memtest;
     bool have_a2a = false;
@@ -83,6 +84,11 @@ static int labels_from_stdin() {
             memset(&r, 0, sizeof(r));
             in >> gpu >> r.tflops_median >> r.verified;
             gemm[gpu] = r;
+        } else if (kind == "gemm_fp8") {
+            int gpu; b200probe_gemm_result_t r;
+            memset(&r, 0, sizeof(r));
+            in >> gpu >> r.tflops_median >> r.verified;
+            gemm_fp8[gpu] = r;
         } else if (kind == "passive") {
             int gpu; b200probe_nvlink_status_t st;
             memset(&st, 0, sizeof(st));
@@ -116,6 +122,7 @@ static int labels_from_stdin() {
     auto merge = [&](const labels::Labels& got) { for (const auto& kv : got) l[kv.first] = kv.second; };
     if (!hbm.empty()) merge(labels::hbm_labels(hbm, th));
     if (!gemm.empty()) merge(labels::gemm_labels(gemm, th));
+    if (!gemm_fp8.empty()) merge(labels::gemm_fp8_labels(gemm_fp8, th));
     merge(labels::nvlink_passive_labels(passive));
     for (const auto& kv : memtest) merge(labels::memtest_labels(kv.first, kv.second));
     if (!memtest.empty()) {

@@ -176,6 +176,26 @@ func GEMM(idx, m, n, k, operands int) (tflops float64, verified bool, err error)
 	return float64(res.tflops_median), res.verified == 1, err
 }
 
+// GEMMFP8 runs the FP8 tensor-core probe (tcgen05.mma kind::f8f6f4, E4M3 operands, bf16 C; 0 = 8192 defaults) and
+// returns median TFLOP/s and the data verdict. operands: 0 = integers in [-8, 7] (C bit-exact against fp64), 1 = Philox
+// U(-1,1) rounded to E4M3 (sampled outputs within tolerance). m and n must be multiples of 256, k a multiple of 128.
+func GEMMFP8(idx, m, n, k, operands int) (tflops float64, verified bool, err error) {
+	runtime.LockOSThread()
+	defer runtime.UnlockOSThread()
+	cfg := C.b200probe_gemm_cfg_t{m: C.int(m), n: C.int(n), k: C.int(k), operands: C.int(operands)}
+	var res C.b200probe_gemm_result_t
+	err = check(C.b200probe_gemm_fp8(C.int(idx), &cfg, &res))
+	return float64(res.tflops_median), res.verified == 1, err
+}
+
+// GEMMFP8Launch queues one E4M3 GEMM on caller-owned device buffers: A [m][k] and B [n][k] E4M3 row-major, C [m][n]
+// bf16, all 16-byte aligned (stream 0 = the default stream).
+func GEMMFP8Launch(ordinal int, a, b, c unsafe.Pointer, m, n, k int, stream unsafe.Pointer) error {
+	runtime.LockOSThread()
+	defer runtime.UnlockOSThread()
+	return check(C.b200probe_gemm_fp8_launch(C.int(ordinal), a, b, c, C.int(m), C.int(n), C.int(k), stream))
+}
+
 // ErrNoMem is B200PROBE_ENOMEM: a device allocation failed because tenants hold the memory. A resource verdict
 // ("inconclusive"), never a health verdict.
 const ErrNoMem = -10

@@ -18,6 +18,7 @@
  *   b200probe_hbm_*         -> NEW: no reference counterpart (SURVEY.md §8a row a11)
  *   b200probe_a2a_*         -> NEW: row a12
  *   b200probe_gemm*         -> NEW: row a13
+ *   b200probe_gemm_fp8*     -> NEW: row a15 (FP8 tensor cores, DESIGN.md §4.5)
  *   b200probe_hbm_memtest,
  *   b200probe_memtest_element,
  *   b200probe_hbm_ecc       -> NEW: HBM integrity (DESIGN.md §4.4)
@@ -398,10 +399,25 @@ int b200probe_gemm_release(int cuda_ordinal);
 int b200probe_gemm_launch(int cuda_ordinal, const void* a, const void* b, void* c,
                           int m, int n, int k, void* stream);
 /* Deterministic bf16 operand generators used by the probe and restated by the oracle.
- * which: bit 0 = matrix (0 = A, 1 = B), bit 1 = operand class (0 EXACT, 1 UNIFORM); dst 16-byte aligned.
+ * which: bit 0 = matrix (0 = A, 1 = B), bit 1 = operand class (0 EXACT, 1 UNIFORM), bit 2 = E4M3 (below); dst 16-byte aligned.
  * b200probe_gemm_operand_bits is the same function for one element on the host (the library's own check uses it). */
 int b200probe_gemm_fill(int cuda_ordinal, void* dst, uint64_t elems, uint32_t seed, int which, void* stream);
 uint16_t b200probe_gemm_operand_bits(uint64_t elem, uint32_t seed, int which);
+
+/* ---- FP8 tensor-core probe (DESIGN.md §4.5): tcgen05.mma kind::f8f6f4, E4M3 x E4M3 -> fp32 -> bf16 --------------------------
+ * b200probe_gemm_fill / b200probe_gemm_operand_bits with bit 2 of `which` set generate E4M3 operands, one byte per element
+ * (dst receives `elems` bytes; operand_bits returns the byte in the low 8 bits):
+ *   EXACT    integers in [-8, 7]: every partial sum is an exact fp32 integer -> C bit-exact against the fp64 contraction
+ *            rounded once to bf16
+ *   UNIFORM  the UNIFORM class's Philox U(-1,1) fp32 values rounded to E4M3 (nearest even); E4M3 products are exact in
+ *            fp32, so the bf16 class's tolerance 2^-8 |ref| + 2^-10 sqrt(K) applies unchanged
+ * b200probe_gemm_fp8 takes the same cfg and result as b200probe_gemm, with the same defaults and verdict rules; m and n must
+ * be multiples of 256 and k a multiple of 128 (else B200PROBE_EINVAL).  It shares the resident arena that
+ * b200probe_gemm_release frees. */
+int b200probe_gemm_fp8(int idx, const b200probe_gemm_cfg_t* cfg, b200probe_gemm_result_t* out);
+/* Resident launch: A [m][k] and B [n][k] E4M3 row-major (C = A * B^T), C [m][n] bf16, 16-byte aligned.  Asynchronous on stream. */
+int b200probe_gemm_fp8_launch(int cuda_ordinal, const void* a, const void* b, void* c,
+                              int m, int n, int k, void* stream);
 
 /* ---- data pattern (closed form shared by kernels, oracle and tests) ----------------------------- */
 /* word i of a buffer:  ((uint32_t)i * 2654435761u) ^ seed ^ (uint32_t)(i >> 32)                   */

@@ -20,6 +20,7 @@ VARIANT_TMA, VARIANT_DIRECT = 0, 1
 A2A_PEER_ALL, A2A_PEER_PAIR, A2A_NCCL, A2A_CE = 0, 1, 2, 3
 PAIR_SHARE, PAIR_ISOLATED, PAIR_STEPPED = 0, 1, 2
 GEMM_EXACT, GEMM_UNIFORM = 0, 1
+GEMM_FILL_E4M3 = 4          # b200probe_gemm_fill / _operand_bits: bit 2 of `which` selects E4M3 operands (one byte per element)
 MEMTEST_VERIFY, MEMTEST_WRITE = 1, 2
 A2A_AUTO, A2A_PULL_TMA, A2A_PUSH_TMA, A2A_PUSH_DIRECT, A2A_PUSH_BUF, A2A_MIX_TMA, A2A_PUSH_STAGGER, A2A_PUSH_SYNC = 0, 1, 2, 3, 4, 5, 6, 7
 A2A_SYNC_BYTES = 4096
@@ -272,6 +273,8 @@ SIGNATURES = {
     "b200probe_gemm_operand_bits": (C.c_uint16, [C.c_uint64, C.c_uint32, C.c_int]),
     "b200probe_gemm_launch": (C.c_int, [C.c_int, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, _vp]),
     "b200probe_gemm_fill": (C.c_int, [C.c_int, _vp, C.c_uint64, C.c_uint32, C.c_int, _vp]),
+    "b200probe_gemm_fp8": (C.c_int, [C.c_int, _P(GemmCfg), _P(GemmResult)]),
+    "b200probe_gemm_fp8_launch": (C.c_int, [C.c_int, _vp, _vp, _vp, C.c_int, C.c_int, C.c_int, _vp]),
     "b200probe_pattern_word": (C.c_uint32, [C.c_uint64, C.c_uint32]),
 }
 

@@ -17,6 +17,8 @@
 //              bit-exact against the fp64 oracle after one bf16 RNE (the probe's default: a health verdict with no tolerance)
 //   1 UNIFORM  SURVEY.md §8d's input class: bf16 U(-1,1) from Philox4x32-10, key (seed, 0); sampled outputs against fp64
 //              dot products within |err| <= 2^-8 |ref| + 2^-10 sqrt(K) (final bf16 rounding + fp32 accumulation allowance)
+// FP8: gemm_e4m3_tn_2cta_512_kernel is the 512 x 256 kernel's body with E4M3 operands (tcgen05.mma kind::f8f6f4, SASS UTCQMMA,
+// K=32 per MMA, 128 elements = the same 128 bytes per k-block) and the same two operand classes in E4M3 (DESIGN.md §4.5).
 #include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
@@ -582,10 +584,37 @@ __device__ __forceinline__ TileCoord tile_coord3(int t, int num_m, int num_n, in
     return {(first_m + in_band % rows) * 4 * BM, (in_band / rows) * BN};
 }
 
+// Operand kinds of the 512 x 256 kernel.  Every k-block is 128 bytes of each operand row (one SWIZZLE_128B atom) and four
+// MMAs 32 bytes apart, so stage sizes, expect_tx counts, shared-memory descriptors and the epilogue are the same for both;
+// the kind differs in the MMA, its instruction descriptor and the elements per k-block (the TMA K coordinate).
+__device__ __forceinline__ void umma_e4m3_2sm(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\t"
+        "setp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::2.kind::f8f6f4 [%0], %1, %2, %3, p;\n\t}" ::"r"(d_tmem),
+        "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
+        : "memory");
+}
+struct OperandBf16 {                                    // kind::f16, M256 N256 K16: 64 bf16 per k-block
+    static constexpr int kKbElems = BK;
+    static constexpr bool kE4m3 = false;
+    static constexpr bool kStagedEpilogue = true;       // has a C tensor map (B200PROBE_GEMM_EPI=1)
+};
+struct OperandE4m3 {                                    // kind::f8f6f4, M256 N256 K32: 128 E4M3 per k-block
+    static constexpr int kKbElems = 128;
+    static constexpr bool kE4m3 = true;
+    static constexpr bool kStagedEpilogue = false;
+    // kind::f8f6f4 instruction descriptor: D = F32 (bit 4), A and B format E4M3 (0 in [7,10) and [10,13)), no negation, both
+    // K-major (bits 15, 16 clear), N>>3 at [17,23), M>>4 at [24,29)
+    static constexpr uint32_t kIdesc = (1u << 4) | (0u << 7) | (0u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)((2 * BM) >> 4) << 24);
+};
+static_assert(OperandE4m3::kKbElems * 1 == BK * 2, "an E4M3 k-block is the same 128 bytes as a bf16 one");
+constexpr GemmTune kShippedTune3{4, 0, 0, 0, 0, 0, 0, 0};   // the 512 x 256 kernel's schedule with every knob at its default
+
 constexpr int NUM_THREADS3 = 384;                       // warps 0-3: TMA producer, MMA issuer, TMEM allocator, idle; warps 4-11: epilogue
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS3, 1)
-gemm_bf16_tn_2cta_512_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, const __grid_constant__ CUtensorMap tma_c,
-                             __nv_bfloat16* __restrict__ C, int M, int N, int K, GemmTune tune) {
+template <class Op>
+__device__ __forceinline__ void gemm_tn_2cta_512(const CUtensorMap* tma_a, const CUtensorMap* tma_b, const CUtensorMap* tma_c,
+                                                 __nv_bfloat16* __restrict__ C, int M, int N, int K, GemmTune tune) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
     uint8_t* smem_a = smem;
@@ -602,14 +631,14 @@ gemm_bf16_tn_2cta_512_kernel(const __grid_constant__ CUtensorMap tma_a, const __
     const uint32_t cta_rank = cluster_ctarank();
     const bool leader = cta_rank == 0;
     // rows past M are zero-filled by the tensor loads and clipped by the tensor stores: any M that is a multiple of 128 works
-    const int num_m = (M + 4 * BM - 1) / (4 * BM), num_n = N / BN, num_tiles = num_m * num_n, num_kb = K / BK;
+    const int num_m = (M + 4 * BM - 1) / (4 * BM), num_n = N / BN, num_tiles = num_m * num_n, num_kb = K / Op::kKbElems;
     // cluster i sits on SMs 2(i-3), 2(i-3)+1 (tools/smid_probe.cu): consecutive pairs are neighbours on the chip already
     const int pair = blockIdx.x >> 1, num_pairs = gridDim.x >> 1;
 
     if (warp == 0 && lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&tma_a) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&tma_b) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)&tma_c) : "memory");
+        asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)tma_a) : "memory");
+        asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)tma_b) : "memory");
+        if constexpr (Op::kStagedEpilogue) asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)tma_c) : "memory");
     }
     if (warp == 1 && lane == 0) {
         for (int s = 0; s < STAGES3; ++s) { mbar_init(smem_u32(&full[s]), 1); mbar_init(smem_u32(&empty[s]), 1); }
@@ -635,9 +664,9 @@ gemm_bf16_tn_2cta_512_kernel(const __grid_constant__ CUtensorMap tma_a, const __
                 const int ti = pair + (int)(gkb / num_kb) * num_pairs;
                 if (ti >= num_tiles) return;
                 const TileCoord pc = tile_coord3(ti, num_m, num_n, tune.group_m);
-                const int k0 = (int)(gkb % num_kb) * BK;
-                tma_prefetch_l2_2d(&tma_a, k0, pc.m0 + (int)cta_rank * 2 * BM);
-                tma_prefetch_l2_2d(&tma_b, k0, pc.n0 + (int)cta_rank * (BN / 2));
+                const int k0 = (int)(gkb % num_kb) * Op::kKbElems;
+                tma_prefetch_l2_2d(tma_a, k0, pc.m0 + (int)cta_rank * 2 * BM);
+                tma_prefetch_l2_2d(tma_b, k0, pc.n0 + (int)cta_rank * (BN / 2));
             };
             long long gkb = 0;
             for (int pf = 0; pf < tune.prefetch; ++pf) prefetch_block(pf);
@@ -649,10 +678,10 @@ gemm_bf16_tn_2cta_512_kernel(const __grid_constant__ CUtensorMap tma_a, const __
                     mbar_wait(smem_u32(&empty[stage]), phase ^ 1);
                     const uint32_t fb = smem_u32(&full[stage]);
                     if (leader) mbar_expect_tx(fb, 2 * STAGE3_BYTES);      // both CTAs' bytes land on the leader's barrier
-                    if (tune.pol_a) tma_load_2d_2sm_hint(smem_u32(smem_a + stage * A3_STAGE_BYTES), &tma_a, fb, kb * BK, my_m, pa);
-                    else tma_load_2d_2sm(smem_u32(smem_a + stage * A3_STAGE_BYTES), &tma_a, fb, kb * BK, my_m);
-                    if (tune.pol_b) tma_load_2d_2sm_hint(smem_u32(smem_b + stage * B3_STAGE_BYTES), &tma_b, fb, kb * BK, my_n, pb);
-                    else tma_load_2d_2sm(smem_u32(smem_b + stage * B3_STAGE_BYTES), &tma_b, fb, kb * BK, my_n);
+                    if (tune.pol_a) tma_load_2d_2sm_hint(smem_u32(smem_a + stage * A3_STAGE_BYTES), tma_a, fb, kb * Op::kKbElems, my_m, pa);
+                    else tma_load_2d_2sm(smem_u32(smem_a + stage * A3_STAGE_BYTES), tma_a, fb, kb * Op::kKbElems, my_m);
+                    if (tune.pol_b) tma_load_2d_2sm_hint(smem_u32(smem_b + stage * B3_STAGE_BYTES), tma_b, fb, kb * Op::kKbElems, my_n, pb);
+                    else tma_load_2d_2sm(smem_u32(smem_b + stage * B3_STAGE_BYTES), tma_b, fb, kb * Op::kKbElems, my_n);
                     if (++stage == STAGES3) { stage = 0; phase ^= 1; }
                 }
             }
@@ -676,7 +705,8 @@ gemm_bf16_tn_2cta_512_kernel(const __grid_constant__ CUtensorMap tma_a, const __
                 const uint64_t b_desc = make_smem_desc(smem_u32(smem_b + stage * B3_STAGE_BYTES));
 #pragma unroll
                 for (int k = 0; k < BK / UMMA_K; ++k)
-                    umma_bf16_2sm(tmem_base + h * BN, a_desc + (uint64_t)(k * 2), b_desc + (uint64_t)(k * 2), kIdesc2, (kb | k) != 0);
+                    if constexpr (Op::kE4m3) umma_e4m3_2sm(tmem_base + h * BN, a_desc + (uint64_t)(k * 2), b_desc + (uint64_t)(k * 2), Op::kIdesc, (kb | k) != 0);
+                    else umma_bf16_2sm(tmem_base + h * BN, a_desc + (uint64_t)(k * 2), b_desc + (uint64_t)(k * 2), kIdesc2, (kb | k) != 0);
             };
             auto wait_full = [&](long long g) {
                 mbar_wait(smem_u32(&full[g % STAGES3]), (uint32_t)((g / STAGES3) & 1));
@@ -726,7 +756,7 @@ gemm_bf16_tn_2cta_512_kernel(const __grid_constant__ CUtensorMap tma_a, const __
                 epilogue_slice_direct(taddr, C + (size_t)row * N + tc.n0, row < M, release);
                 continue;
             }
-            epilogue_slice32(taddr, stage, ubuf, &tma_c, row0, tc.n0, lane, [&]() {
+            epilogue_slice32(taddr, stage, ubuf, tma_c, row0, tc.n0, lane, [&]() {
                 tc_fence_before();                         // this warp's slice is in registers: 8 such arrivals free accumulator h
                 __syncwarp();
                 if (lane == 0) mbar_arrive_leader(tempty_bar);
@@ -740,6 +770,17 @@ gemm_bf16_tn_2cta_512_kernel(const __grid_constant__ CUtensorMap tma_a, const __
         tc_fence_after();
         asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(TMEM_COLS) : "memory");
     }
+}
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS3, 1)
+gemm_bf16_tn_2cta_512_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, const __grid_constant__ CUtensorMap tma_c,
+                             __nv_bfloat16* __restrict__ C, int M, int N, int K, GemmTune tune) {
+    gemm_tn_2cta_512<OperandBf16>(&tma_a, &tma_b, &tma_c, C, M, N, K, tune);
+}
+// A [M][K] and B [N][K] E4M3, C [M][N] bf16: the shipped schedule, no tuning knobs (epilogue straight from registers, no C map)
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS3, 1)
+gemm_e4m3_tn_2cta_512_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b, __nv_bfloat16* __restrict__ C, int M, int N,
+                             int K) {
+    gemm_tn_2cta_512<OperandE4m3>(&tma_a, &tma_b, nullptr, C, M, N, K, kShippedTune3);
 }
 
 // `which`: bit 0 = matrix (0 A, 1 B), bit 1 = operand class (0 EXACT k/128, 1 UNIFORM Philox U(-1,1))
@@ -764,6 +805,35 @@ __global__ void gemm_fill_kernel(uint16_t* dst, uint64_t elems, uint32_t seed, i
     } else {
         for (; i < elems; i += stride) dst[i] = b200_gemm_elem_bits(i, seed, which);
     }
+}
+
+// E4M3 operands (b200probe_gemm_fill with bit 2 of `which` set): one byte per element, four elements (one Philox block of the
+// UNIFORM class) per 4-byte store, rounded by the hardware conversion (the host twin is b200_e4m3_rne)
+__device__ __forceinline__ uint32_t e4m3x4(float x0, float x1, float x2, float x3) {
+    uint16_t lo, hi;
+    asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(lo) : "f"(x1), "f"(x0));       // x0 -> the low byte
+    asm("cvt.rn.satfinite.e4m3x2.f32 %0, %1, %2;" : "=h"(hi) : "f"(x3), "f"(x2));
+    return (uint32_t)lo | ((uint32_t)hi << 16);
+}
+__global__ void gemm_fill_e4m3_kernel(uint8_t* dst, uint64_t elems, uint32_t seed, int which) {
+    const uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const uint64_t stride = (uint64_t)gridDim.x * blockDim.x;
+    const int mat = which & 1, uniform = (which >> 1) & 1;
+    const uint64_t nblk = elems >> 2;
+    for (uint64_t b = i; b < nblk; b += stride) {
+        float x[4];
+        if (uniform) {
+            uint32_t r[4];
+            b200_philox4x32_10((uint32_t)b, (uint32_t)(b >> 32), (uint32_t)mat, 0u, seed, 0u, r);
+#pragma unroll
+            for (int j = 0; j < 4; ++j) x[j] = (float)(r[j] >> 8) * (1.0f / 8388608.0f) - 1.0f;
+        } else {
+#pragma unroll
+            for (int j = 0; j < 4; ++j) x[j] = b200_gemm_e4m3_value(4 * b + j, seed, mat, 0);
+        }
+        *reinterpret_cast<uint32_t*>(dst + 4 * b) = e4m3x4(x[0], x[1], x[2], x[3]);
+    }
+    for (uint64_t e = (nblk << 2) + i; e < elems; e += stride) dst[e] = (uint8_t)e4m3x4(b200_gemm_e4m3_value(e, seed, mat, uniform), 0.f, 0.f, 0.f);
 }
 
 __global__ void gather_kernel(const uint16_t* c, const uint64_t* idx, uint16_t* out, int n) {
@@ -791,21 +861,25 @@ int get_encode(EncodeTiledFn* fn) {
     return 0;
 }
 
-// [rows][inner] bf16 row-major -> box {64 (inner), box_rows}, 128B swizzle.  Operands: inner = K; C: inner = N.
-// box_cols = 32 selects the 64-byte-swizzled map of the 32-column epilogue units.
-int make_map(CUtensorMap* map, const void* base, int rows, int inner, int box_rows, int box_cols = BK) {
+// [rows][inner] row-major -> box {box_cols (inner), box_rows}, 128B swizzle.  Operands: inner = K; C: inner = N.
+// bf16 (the default): box_cols = 64 is one 128-byte row; box_cols = 32 selects the 64-byte-swizzled map of the 32-column
+// epilogue units.  E4M3 operands: CU_TENSOR_MAP_DATA_TYPE_UINT8, 1 byte, box_cols = 128.  The L2 promotion experiment
+// (B200PROBE_GEMM_L2_PROMOTION) belongs to the bf16 kernels: other element types get the default 256 B.
+int make_map(CUtensorMap* map, const void* base, int rows, int inner, int box_rows, int box_cols = BK,
+             CUtensorMapDataType dtype = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, int elem_bytes = 2) {
     EncodeTiledFn enc = nullptr;
     int rc = get_encode(&enc);
     if (rc) return rc;
     cuuint64_t dims[2] = {(cuuint64_t)inner, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)inner * 2};
+    cuuint64_t strides[1] = {(cuuint64_t)inner * elem_bytes};
     cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
     cuuint32_t estr[2] = {1, 1};
     static const int l2prom = [] { const char* e = getenv("B200PROBE_GEMM_L2_PROMOTION"); return e ? atoi(e) : 256; }();      // experiments: 0, 64, 128, 256
-    const CUtensorMapL2promotion prom = l2prom == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : l2prom == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-                                      : l2prom == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
-    CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                     box_cols == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, prom, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    const int l2 = dtype == CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 ? l2prom : 256;
+    const CUtensorMapL2promotion prom = l2 == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : l2 == 64 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
+                                      : l2 == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
+    CUresult r = enc(map, dtype, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                     box_cols * elem_bytes == 64 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B, prom, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) { b200::set_error("cuTensorMapEncodeTiled failed: CUresult %d", (int)r); return B200PROBE_CUDA_BASE + 1; }
     return 0;
 }
@@ -814,6 +888,14 @@ static_assert(EPI_UNIT_COLS == BK, "the C map reuses the operands' 64-element (1
 int check_shape(int m, int n, int k) {
     if (m <= 0 || n <= 0 || k <= 0 || m % BM || n % BN || k % BK) {
         b200::set_error("gemm: m,n,k must be positive multiples of %d,%d,%d (got %d,%d,%d)", BM, BN, BK, m, n, k);
+        return B200PROBE_EINVAL;
+    }
+    return 0;
+}
+// the E4M3 kernel: CTA pairs of 256 rows, k-blocks of 128 elements
+int check_shape_fp8(int m, int n, int k) {
+    if (m <= 0 || n <= 0 || k <= 0 || m % (2 * BM) || n % BN || k % OperandE4m3::kKbElems) {
+        b200::set_error("gemm_fp8: m,n,k must be positive multiples of %d,%d,%d (got %d,%d,%d)", 2 * BM, BN, OperandE4m3::kKbElems, m, n, k);
         return B200PROBE_EINVAL;
     }
     return 0;
@@ -837,9 +919,16 @@ uint16_t float_to_bf16_rne(float f) {
     uint32_t r = 0x7fffu + ((u >> 16) & 1u);
     return (uint16_t)((u + r) >> 16);
 }
+double e4m3_bits_to_double(uint8_t v) {
+    const int e = (v >> 3) & 15, m = v & 7;
+    if (e == 15 && m == 7) return NAN;
+    const double mag = e ? ldexp(8 + m, e - 10) : ldexp(m, -9);      // (1 + m/8) 2^(e-7), subnormal m/8 2^-6
+    return (v & 0x80) ? -mag : mag;
+}
 
-// Per-device resident arena (like hbm_sweep.cu's): operands stay filled between calls with the same shape, seed and
-// operand class — the daemon probes periodically, and 384 MiB of cudaMalloc + two fills cost more than the ten timed GEMMs.
+// Per-device resident arena (like hbm_sweep.cu's): operands stay filled between calls with the same shape, seed, operand
+// class and element type — the daemon probes periodically, and 384 MiB of cudaMalloc + two fills cost more than the ten
+// timed GEMMs.  Operand buffers are sized for bf16; E4M3 operands use the first half of them.
 struct GemmArena {
     pthread_mutex_t mu = PTHREAD_MUTEX_INITIALIZER;
     void *a = nullptr, *b = nullptr, *c = nullptr, *idx = nullptr, *out = nullptr;
@@ -847,6 +936,7 @@ struct GemmArena {
     cudaStream_t stream = nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
     int m = 0, n = 0, k = 0, operands = -1, samples_cap = 0;
+    int e4m3 = -1;                                          // element type of the filled operands: 0 bf16, 1 E4M3
     uint32_t seed = 0;
     bool filled = false;
 };
@@ -864,7 +954,7 @@ void gemm_arena_free(GemmArena& g) {
     if (g.stream) cudaStreamDestroy(g.stream);
     g.a = g.b = g.c = g.idx = g.out = nullptr;
     g.partials = nullptr; g.e0 = g.e1 = nullptr; g.stream = nullptr;
-    g.m = g.n = g.k = 0; g.operands = -1; g.samples_cap = 0; g.filled = false;
+    g.m = g.n = g.k = 0; g.operands = -1; g.e4m3 = -1; g.samples_cap = 0; g.filled = false;
 }
 
 
@@ -911,14 +1001,16 @@ int b200probe_gemm_fill(int ordinal, void* dst, uint64_t elems, uint32_t seed, i
     b200::DevProps props;
     int rc = b200::device_props(ordinal, &props);
     if (rc) return rc;
-    if (!dst || which < 0 || which > 3 || (((uintptr_t)dst) & 15)) return B200PROBE_EINVAL;
+    if (!dst || which < 0 || which > 7 || (((uintptr_t)dst) & 15)) return B200PROBE_EINVAL;
     B200_CUDA_TRY(cudaSetDevice(ordinal));
-    if (elems) gemm_fill_kernel<<<props.sms * 8, 256, 0, (cudaStream_t)stream>>>((uint16_t*)dst, elems, seed, which);
+    if (elems && (which & 4)) gemm_fill_e4m3_kernel<<<props.sms * 8, 256, 0, (cudaStream_t)stream>>>((uint8_t*)dst, elems, seed, which & 3);
+    else if (elems) gemm_fill_kernel<<<props.sms * 8, 256, 0, (cudaStream_t)stream>>>((uint16_t*)dst, elems, seed, which);
     B200_CUDA_TRY(cudaGetLastError());
     return 0;
 }
 
 uint16_t b200probe_gemm_operand_bits(uint64_t elem, uint32_t seed, int which) {
+    if (which & 4) return b200_e4m3_rne(b200_gemm_e4m3_value(elem, seed, which & 1, (which >> 1) & 1));
     return (which & 2) ? b200_gemm_uniform_bits(elem, seed, which & 1) : b200_gemm_elem_bits(elem, seed, which & 1);
 }
 
@@ -952,7 +1044,7 @@ int b200probe_gemm_launch(int ordinal, const void* a, const void* b, void* c, in
         B200_CUDA_TRY(cudaFuncSetAttribute(gemm_bf16_tn_2cta_512_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM3_BYTES));
         const int tiles = ((m + 4 * BM - 1) / (4 * BM)) * (n / BN);
         const int pairs = std::min(tiles, props.sms / 2);
-        GemmTune tune{4, 0, 0, 0, 0, 0, 0, 0};  // bands of 4 x 512 rows (the same 2048 rows as the 256 x 256 kernel's bands)
+        GemmTune tune = kShippedTune3;          // bands of 4 x 512 rows (the same 2048 rows as the 256 x 256 kernel's bands)
         if (const char* e = getenv("B200PROBE_GEMM_PREFETCH")) { int v = atoi(e); if (v >= 0 && v <= 64) tune.prefetch = v; }
         if (const char* e = getenv("B200PROBE_GEMM_EXPT")) tune.expt = atoi(e);
         if (const char* e = getenv("B200PROBE_GEMM_EPI")) tune.epi = atoi(e);
@@ -982,6 +1074,27 @@ int b200probe_gemm_launch(int ordinal, const void* a, const void* b, void* c, in
     return 0;
 }
 
+int b200probe_gemm_fp8_launch(int ordinal, const void* a, const void* b, void* c, int m, int n, int k, void* stream) {
+    b200::DevProps props;
+    int rc = b200::device_props(ordinal, &props);
+    if (rc) return rc;
+    rc = check_shape_fp8(m, n, k);
+    if (rc) return rc;
+    if (!a || !b || !c || (((uintptr_t)a | (uintptr_t)b | (uintptr_t)c) & 15)) { b200::set_error("gemm_fp8: operands must be 16-byte aligned device pointers"); return B200PROBE_EINVAL; }
+    B200_CUDA_TRY(cudaSetDevice(ordinal));
+    CUtensorMap ma, mb;
+    rc = make_map(&ma, a, m, k, 2 * BM, OperandE4m3::kKbElems, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1);
+    if (rc) return rc;
+    rc = make_map(&mb, b, n, k, BN / 2, OperandE4m3::kKbElems, CU_TENSOR_MAP_DATA_TYPE_UINT8, 1);
+    if (rc) return rc;
+    B200_CUDA_TRY(cudaFuncSetAttribute(gemm_e4m3_tn_2cta_512_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM3_BYTES));
+    const int tiles = ((m + 4 * BM - 1) / (4 * BM)) * (n / BN);
+    const int pairs = std::min(tiles, props.sms / 2);
+    gemm_e4m3_tn_2cta_512_kernel<<<2 * pairs, NUM_THREADS3, SMEM3_BYTES, (cudaStream_t)stream>>>(ma, mb, (__nv_bfloat16*)c, m, n, k);
+    B200_CUDA_TRY(cudaGetLastError());
+    return 0;
+}
+
 int b200probe_gemm_release(int ordinal) {
     if (ordinal < 0 || ordinal >= B200PROBE_MAX_DEVICES) return B200PROBE_ERANGE;
     GemmArena& g = g_gemm[ordinal];
@@ -990,24 +1103,31 @@ int b200probe_gemm_release(int ordinal) {
     return 0;
 }
 
-static int gemm_locked(int ordinal, GemmArena& g, const b200probe_gemm_cfg_t& cfg, b200probe_gemm_result_t* out) {
+// e4m3 = 0: the bf16 kernels (b200probe_gemm), 1: the E4M3 kernel (b200probe_gemm_fp8); the same protocol and verdict rules
+static int gemm_locked(int ordinal, GemmArena& g, const b200probe_gemm_cfg_t& cfg, int e4m3, b200probe_gemm_result_t* out) {
     const int M = cfg.m, N = cfg.n, K = cfg.k, S = cfg.samples;
     const int cls = cfg.operands;
+    const int kind = (e4m3 ? 4 : 0) | (cls << 1);                   // b200probe_gemm_fill's `which` without the matrix bit
+    auto launch = [&]() { return e4m3 ? b200probe_gemm_fp8_launch(ordinal, g.a, g.b, g.c, M, N, K, g.stream) : b200probe_gemm_launch(ordinal, g.a, g.b, g.c, M, N, K, g.stream); };
+    auto value = [&](uint64_t e, int mat) {
+        const uint16_t v = b200probe_gemm_operand_bits(e, cfg.seed, kind | mat);
+        return e4m3 ? e4m3_bits_to_double((uint8_t)v) : (double)bf16_bits_to_float(v);
+    };
     int rc = gemm_arena_reserve(g, M, N, K, S);
     if (rc) return rc;
-    if (!g.filled || g.seed != cfg.seed || g.operands != cls) {
-        rc = b200probe_gemm_fill(ordinal, g.a, (uint64_t)M * K, cfg.seed, 0 | (cls << 1), g.stream);
+    if (!g.filled || g.seed != cfg.seed || g.operands != cls || g.e4m3 != e4m3) {
+        rc = b200probe_gemm_fill(ordinal, g.a, (uint64_t)M * K, cfg.seed, kind | 0, g.stream);
         if (rc) return rc;
-        rc = b200probe_gemm_fill(ordinal, g.b, (uint64_t)N * K, cfg.seed, 1 | (cls << 1), g.stream);
+        rc = b200probe_gemm_fill(ordinal, g.b, (uint64_t)N * K, cfg.seed, kind | 1, g.stream);
         if (rc) return rc;
-        g.filled = true; g.seed = cfg.seed; g.operands = cls;
+        g.filled = true; g.seed = cfg.seed; g.operands = cls; g.e4m3 = e4m3;
     }
     B200_CUDA_TRY(cudaMemsetAsync(g.c, 0xFF, (size_t)M * N * 2, g.stream));      // poison: a tile the kernel skipped cannot pass the check
 
     std::vector<float> ms((size_t)cfg.reps);
     for (int it = -cfg.warmup; it < cfg.reps; ++it) {
         if (it >= 0) B200_CUDA_TRY(cudaEventRecord(g.e0, g.stream));
-        rc = b200probe_gemm_launch(ordinal, g.a, g.b, g.c, M, N, K, g.stream);
+        rc = launch();
         if (rc) return rc;
         if (it >= 0) {
             B200_CUDA_TRY(cudaEventRecord(g.e1, g.stream));
@@ -1030,7 +1150,7 @@ static int gemm_locked(int ordinal, GemmArena& g, const b200probe_gemm_cfg_t& cf
             float t;
             B200_CUDA_TRY(cudaEventRecord(g.e0, g.stream));
             for (int i = 0; i < batch; ++i) {
-                rc = b200probe_gemm_launch(ordinal, g.a, g.b, g.c, M, N, K, g.stream);
+                rc = launch();
                 if (rc) return rc;
             }
             B200_CUDA_TRY(cudaEventRecord(g.e1, g.stream));
@@ -1071,8 +1191,7 @@ static int gemm_locked(int ordinal, GemmArena& g, const b200probe_gemm_cfg_t& cf
         const uint64_t r = idxs[i] / N, c = idxs[i] % N;
         double acc = 0;
         for (int k = 0; k < K; ++k)
-            acc += (double)bf16_bits_to_float(b200probe_gemm_operand_bits(r * K + k, cfg.seed, 0 | (cls << 1))) *
-                   (double)bf16_bits_to_float(b200probe_gemm_operand_bits(c * K + k, cfg.seed, 1 | (cls << 1)));
+            acc += value(r * K + k, 0) * value(c * K + k, 1);
         const double gotf = bf16_bits_to_float(got[i]);
         const double err = fabs(gotf - acc);
         max_abs = std::max(max_abs, err);
@@ -1089,14 +1208,14 @@ static int gemm_locked(int ordinal, GemmArena& g, const b200probe_gemm_cfg_t& cf
     out->max_abs_err = max_abs; out->max_rel_err = max_rel; out->max_err_over_tol = max_over_tol;
     out->verified = bad == 0 ? 1 : 0;
     if (bad) {
-        b200::set_error("gemm: %d of %d sampled outputs %s (max abs err %g)", bad, S,
+        b200::set_error("%s: %d of %d sampled outputs %s (max abs err %g)", e4m3 ? "gemm_fp8" : "gemm", bad, S,
                         cls == B200PROBE_GEMM_OPERANDS_EXACT ? "differ from the fp64 contraction rounded to bf16" : "are outside 2^-8|ref| + 2^-10 sqrt(K) of the fp64 contraction", max_abs);
         return B200PROBE_EMISMATCH;
     }
     return 0;
 }
 
-int b200probe_gemm(int idx, const b200probe_gemm_cfg_t* cfg_in, b200probe_gemm_result_t* out) {
+static int gemm_entry(int idx, const b200probe_gemm_cfg_t* cfg_in, int e4m3, b200probe_gemm_result_t* out) {
     if (!out) return B200PROBE_EINVAL;
     int ordinal = -1;
     int rc = b200::cuda_ordinal_of(idx, &ordinal);
@@ -1116,7 +1235,7 @@ int b200probe_gemm(int idx, const b200probe_gemm_cfg_t* cfg_in, b200probe_gemm_r
     if (!cfg.samples) cfg.samples = 1024;
     if (cfg.samples < 1 || cfg.samples > (1 << 20)) { b200::set_error("gemm: samples out of range"); return B200PROBE_EINVAL; }
     if (cfg.operands != B200PROBE_GEMM_OPERANDS_EXACT && cfg.operands != B200PROBE_GEMM_OPERANDS_UNIFORM) { b200::set_error("gemm: unknown operand class %d", cfg.operands); return B200PROBE_EINVAL; }
-    rc = check_shape(cfg.m, cfg.n, cfg.k);
+    rc = e4m3 ? check_shape_fp8(cfg.m, cfg.n, cfg.k) : check_shape(cfg.m, cfg.n, cfg.k);
     if (rc) return rc;
     memset(out, 0, sizeof(*out));
     out->m = cfg.m; out->n = cfg.n; out->k = cfg.k;
@@ -1125,9 +1244,13 @@ int b200probe_gemm(int idx, const b200probe_gemm_cfg_t* cfg_in, b200probe_gemm_r
     B200_CUDA_TRY(cudaSetDevice(ordinal));
     GemmArena& g = g_gemm[ordinal];
     GemmLock lock(g);
-    rc = gemm_locked(ordinal, g, cfg, out);
+    rc = gemm_locked(ordinal, g, cfg, e4m3, out);
     if (rc && rc != B200PROBE_EMISMATCH) gemm_arena_free(g);      // unknown state after a CUDA error / failed allocation: start over next time
     return rc;
 }
+
+int b200probe_gemm(int idx, const b200probe_gemm_cfg_t* cfg_in, b200probe_gemm_result_t* out) { return gemm_entry(idx, cfg_in, 0, out); }
+
+int b200probe_gemm_fp8(int idx, const b200probe_gemm_cfg_t* cfg_in, b200probe_gemm_result_t* out) { return gemm_entry(idx, cfg_in, 1, out); }
 
 }  // extern "C"

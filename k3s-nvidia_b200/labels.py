@@ -54,6 +54,9 @@ NVLINK_HEALTHY_GBS = 692.0       # this repo's push kernel with all 18 links up,
 NVLINK_HEALTHY_GBS_BOX = 700.0   # G > 2: one peer per step with the step barrier (profiles/a2a_sync_relaxed_r01_g8.txt: 701 at every GPU)
 GEMM_NOMINAL_TFLOPS = 2250.0
 GEMM_MEASURED_TFLOPS = 1670.2
+# cuBLASLt FP8 (torch._scaled_mm, E4M3 x E4M3, scales 1.0, bf16 out) at 8192^3, burst median on a B200 at its 1000 W power
+# limit, EXACT operands (profiles/gemm_fp8_bench_r01.txt): the pool figure of the FP8 probe until a node has calibrated its own
+GEMM_FP8_MEASURED_TFLOPS = 3268.0
 
 _LABEL_VALUE = re.compile(r"^(([A-Za-z0-9][-A-Za-z0-9_.]*)?[A-Za-z0-9])?$")
 _LABEL_NAME = re.compile(r"^([A-Za-z0-9][-A-Za-z0-9_.]*)?[A-Za-z0-9]$")
@@ -73,6 +76,7 @@ class Thresholds:
     # number of GPUs exchanged (0 = derive from G when the labels are made; B200PROBE_NVLINK_MIN_GBS pins it)
     nvlink_min_gbs: float = field(default_factory=lambda: _env_float("B200PROBE_NVLINK_MIN_GBS", 0.0))
     gemm_min_tflops: float = field(default_factory=lambda: _env_float("B200PROBE_GEMM_MIN_TFLOPS", 0.70 * GEMM_MEASURED_TFLOPS))
+    gemm_fp8_min_tflops: float = field(default_factory=lambda: _env_float("B200PROBE_GEMM_FP8_MIN_TFLOPS", 0.70 * GEMM_FP8_MEASURED_TFLOPS))
     verdict_min_bytes: int = 256 << 20        # sizes below L2 are cache-resident: never used for the verdict
 
 
@@ -195,6 +199,25 @@ def gemm_labels(per_gpu: Dict[int, object], th: Thresholds) -> Dict[str, str]:
     return out
 
 
+def gemm_fp8_labels(per_gpu: Dict[int, object], th: Thresholds) -> Dict[str, str]:
+    """The FP8 tensor-core probe (E4M3, tcgen05.mma kind::f8f6f4): the bf16 GEMM's rules on its own keys and threshold."""
+    out: Dict[str, str] = {}
+    all_ok = True
+    for idx, r in sorted(per_gpu.items()):
+        ok = r.verified == 1 and r.tflops_median >= th.gemm_fp8_min_tflops
+        out[f"{PREFIX}gpu{idx}.gemm-fp8-tflops"] = str(int(round(r.tflops_median)))
+        out[f"{PREFIX}gpu{idx}.gemm-fp8-data-ok"] = _b(r.verified == 1)
+        out[f"{PREFIX}gpu{idx}.gemm-fp8-healthy"] = _b(ok)
+        all_ok = all_ok and ok
+    out[f"{PREFIX}gemm-fp8-healthy"] = _b(all_ok and bool(per_gpu))
+    return out
+
+
+def gemm_fp8_enabled() -> bool:
+    """B200PROBE_GEMM_FP8=1: every idle GPU also runs the FP8 tensor-core probe; unset or 0 = off."""
+    return os.environ.get("B200PROBE_GEMM_FP8", "") not in ("", "0")
+
+
 def memtest_labels(idx: int, r) -> Dict[str, str]:
     """r: probe.MemtestReport of GPU idx.  The verdict fails on a mismatching word, on uncorrected ECC errors during the
     run and on a failed row remap.  Corrected errors and a pending remap are published only: ECC fixed the data, and a
@@ -223,7 +246,8 @@ def gate_label(labels: Dict[str, str]) -> Dict[str, str]:
     """The one label manifests select on: every probe that has a verdict is healthy.  No verdict at all (every GPU
     busy since the daemon started) -> no gate label: unknown is not healthy."""
     parts = [v for k, v in labels.items()
-             if k in (f"{PREFIX}hbm-healthy", f"{PREFIX}nvlink-healthy", f"{PREFIX}gemm-healthy", f"{PREFIX}hbm-memtest-healthy")]
+             if k in (f"{PREFIX}hbm-healthy", f"{PREFIX}nvlink-healthy", f"{PREFIX}gemm-healthy", f"{PREFIX}hbm-memtest-healthy",
+                      f"{PREFIX}gemm-fp8-healthy")]
     return {f"{PREFIX}healthy": _b(all(v == "true" for v in parts))} if parts else {}
 
 
@@ -366,6 +390,7 @@ class ActiveProbeRunner:
         self.th = thresholds or Thresholds()
         self._explicit_hbm_gate = thresholds is not None or "B200PROBE_HBM_MIN_GBS" in os.environ
         self._explicit_gemm_gate = thresholds is not None or "B200PROBE_GEMM_MIN_TFLOPS" in os.environ
+        self._explicit_gemm_fp8_gate = thresholds is not None or "B200PROBE_GEMM_FP8_MIN_TFLOPS" in os.environ
         self.hbm_kwargs = hbm_kwargs or dict(min_bytes=1 << 28, max_bytes=1 << 30, warmup=2, reps=5, verify=1)
         self.run_nvlink = run_nvlink
         self.run_gemm = run_gemm
@@ -464,6 +489,33 @@ class ActiveProbeRunner:
                 labels.update({k: v for k, v in got.items() if _GPU_KEY.match(k)})
                 if got.get(f"{PREFIX}gpu{idx}.gemm-healthy") == "true":
                     self.cal.offer(f"gemm-tflops.{uuid}", r.tflops_median, GEMM_MEASURED_TFLOPS)
+        if gemm_fp8_enabled():
+            for d in infos:
+                if state[d.index] != "probed":
+                    continue
+                try:
+                    r = self.probe.gemm_fp8(d.index, warmup=2, reps=5)
+                except ProbeError as e:
+                    if e.rc == ENOMEM:
+                        state[d.index] = "no-memory"
+                        log.warning("GPU %d: no device memory for the FP8 GEMM probe (tenants hold it): inconclusive", d.index)
+                        continue
+                    log.error("FP8 GEMM probe failed on GPU %d: %s", d.index, e)
+                    labels[f"{PREFIX}gpu{d.index}.gemm-fp8-healthy"] = "false"
+                    continue
+                except Exception as e:  # noqa: BLE001
+                    log.error("FP8 GEMM probe failed on GPU %d: %s", d.index, e)
+                    labels[f"{PREFIX}gpu{d.index}.gemm-fp8-healthy"] = "false"
+                    continue
+                uuid = infos[d.index].uuid
+                th = self.th
+                if not self._explicit_gemm_fp8_gate:
+                    th = Thresholds(hbm_min_gbs=self.th.hbm_min_gbs, nvlink_min_gbs=self.th.nvlink_min_gbs, gemm_min_tflops=self.th.gemm_min_tflops,
+                                    gemm_fp8_min_tflops=0.70 * self.cal.get(f"gemm-fp8-tflops.{uuid}", GEMM_FP8_MEASURED_TFLOPS))
+                got = gemm_fp8_labels({d.index: r}, th)
+                labels.update({k: v for k, v in got.items() if _GPU_KEY.match(k)})
+                if got.get(f"{PREFIX}gpu{d.index}.gemm-fp8-healthy") == "true":
+                    self.cal.offer(f"gemm-fp8-tflops.{uuid}", r.tflops_median, GEMM_FP8_MEASURED_TFLOPS)
         fraction = memtest_fraction()
         if fraction > 0:
             for d in infos:
@@ -489,6 +541,7 @@ class ActiveProbeRunner:
                 self._carry(labels, d.index, "gemm-")
         self._aggregate(labels, "hbm-healthy")
         self._aggregate(labels, "hbm-memtest-healthy")
+        self._aggregate(labels, "gemm-fp8-healthy")
         if self.run_gemm:
             self._aggregate(labels, "gemm-healthy")
         copies = [float(v) for k, v in labels.items() if (m := _GPU_KEY.match(k)) and m.group(2) == "hbm-copy-gbs"]

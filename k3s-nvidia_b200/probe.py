@@ -328,6 +328,22 @@ class Probe:
         self._check(rc, "gemm")
         return rep
 
+    def gemm_fp8(self, idx: int = 0, *, m=0, n=0, k=0, warmup=0, reps=0, seed=0xB200, samples=0, sustain_seconds=0.0,
+                 operands=L.GEMM_EXACT) -> GemmReport:
+        """The FP8 tensor-core probe: E4M3 operands through tcgen05.mma kind::f8f6f4, bf16 C, with gemm()'s protocol and
+        verdict rules.  m and n must be multiples of 256, k a multiple of 128."""
+        cfg = L.GemmCfg(m, n, k, warmup, reps, seed, samples, operands, sustain_seconds)
+        r = L.GemmResult()
+        rc = self.lib.b200probe_gemm_fp8(idx, C.byref(cfg), C.byref(r))
+        rep = GemmReport(r.m, r.n, r.k, r.ms_median, r.ms_best, r.tflops_median, r.tflops_best, r.tflops_sustained,
+                         r.max_abs_err, r.max_rel_err, r.samples, r.bad, r.c_sum64, r.c_xor32, r.verified, r.operands, r.max_err_over_tol)
+        self._check(rc, "gemm_fp8")
+        return rep
+
+    def gemm_fp8_launch(self, ordinal: int, a: int, b: int, c: int, m: int, n: int, k: int, stream=None) -> None:
+        """One asynchronous E4M3 GEMM on device buffers: A [m][k], B [n][k] E4M3 row-major, C [m][n] bf16."""
+        self._check(self.lib.b200probe_gemm_fp8_launch(ordinal, a, b, c, m, n, k, stream), "gemm_fp8_launch")
+
     def release(self, ordinals: Sequence[int] = ()) -> None:
         """Free every resident probe arena (HBM, GEMM per listed CUDA ordinal; the exchange context): what the plugin
         does after a probe round, so the daemon holds no device memory while tenants run."""
